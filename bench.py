@@ -14,7 +14,11 @@ peer-memory stores over NVLink from a kernel of libmbcol.so into rank 0's window
 through ctypes); torch.distributed (NCCL) only carries the 64-byte IPC handle, the barriers and the max-over-ranks time.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload auto|c2|c5] [--rows R] [--impl ours|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+
+`--dump-outputs DIR` (one GPU) writes what the last timed step returned as .npy files, so that two builds can be compared
+output for output on the same seeded table.
 
 `--impl reference` times the reference's CPU algorithm (oracle/: the literal C++ restatement; the Java original cannot
 run here -- no JDK in the image, probed at start) on the box's host cores.  Prints ONE JSON line on rank 0.
@@ -47,6 +51,8 @@ ROW_BYTES_OUT = 36                                       # 8 B position + 28 B p
 
 C5_DESCS = [(1, 4)] * 5 + [(2, 4)] * 2 + [(0, 16)]       # I1..I5, R1, R2, S
 C5_AGGS = [(0, 0), (1, 1), (1, 5), (2, 0), (3, 0)]       # COUNT, SUM(I2), SUM(R1), MIN(I1), MAX(I1)
+
+DUMP_BYTES = 64_000_000                                  # --dump-outputs: size limit of all files of one dump
 
 
 def pred_terms(term_cls, sel: float, int_col: int, real_col: int):
@@ -346,15 +352,18 @@ def run_ours(args, rank: int, local_rank: int, world: int):
         for res in results:
             res.close()
 
-    def read_previous(record=False):
+    def read_previous(record=False, keep=False):
         """N=1: the host reads the counts of the PREVIOUS step (and frees its results) after this step's scans are queued, so
-        the GPU is not idle while the host waits and launches; every step's results are read inside the timed region."""
+        the GPU is not idle while the host waits and launches; every step's results are read inside the timed region.
+        keep: the results are returned to the caller instead of freed."""
         results = list(pending)
         pending.clear()
         for s, res in zip(wl.sels, results):                        # the host reads every count (this is the wait)
             counts[s] = res.count
             if record:
                 kernel_ms[s].append(res.kernel_ms)
+        if keep:
+            return results
         for res in results:
             res.close()
 
@@ -391,9 +400,13 @@ def run_ours(args, rank: int, local_rank: int, world: int):
     if world > 1:
         exchange_previous(record=True)                              # the last step's exchange is inside the timed region
     else:
-        read_previous(record=True)                                  # ... and so is the read of the last step's results
+        last = read_previous(record=True, keep=bool(args.dump_outputs))   # ... and so is the read of the last step's results
     e1.record(stream)
     barrier()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, wl, last, dev)
+        for res in last:
+            res.close()
     ms = e0.elapsed_time(e1)
     launches = ctx.kernel_launches - launches0
     tmax = torch.tensor([ms], dtype=torch.float64, device=dev)
@@ -610,6 +623,44 @@ class _CudaArray:
         self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (ptr, False), "version": 3}
 
 
+def dump_outputs(out_dir, wl, results, dev):
+    """Write what a caller of the timed path received from its last step to out_dir, per query (file prefix sel<s>_): the
+    positions, every projected column (col<c>) and the aggregates.  Positions, integers and aggregates are stored as
+    float64, reals and string bytes as float32.  An aggregate without a value (MIN / MAX of no rows) is NaN.  A query with
+    more rows than its share of DUMP_BYTES is represented by a sample: sorted row indices drawn with a fixed seed, the same
+    on every run that returns as many rows, so that dumps of two builds compare element for element."""
+    import torch
+    from mbcol import _native as N
+
+    def rows_of(ptr, stride, n, idx):
+        """Rows idx of a device array of n rows of `stride` bytes, as a host uint8 array of shape (len(idx), stride)."""
+        if n == 0:
+            return np.zeros((0, stride), dtype=np.uint8)
+        rows = torch.as_tensor(_CudaArray(ptr, n * stride), device=dev).view(n, stride)
+        return rows[torch.from_numpy(idx).to(dev)].cpu().numpy()
+
+    os.makedirs(out_dir, exist_ok=True)
+    row_bytes = 8 + sum(4 * w if t == N.ATTR_STRING else 8 if t == N.ATTR_INTEGER else 4 for t, w in (wl.descs[c] for c in wl.proj))
+    cap = (DUMP_BYTES - (1 << 16)) // (len(wl.sels) * row_bytes)      # 64 KB left for the .npy headers and the aggregates
+    for s, res in zip(wl.sels, results):
+        n = res.count
+        idx = np.arange(n) if n <= cap else np.sort(np.random.default_rng(SEED).choice(n, cap, replace=False))
+        out = {"positions": rows_of(res.device_pointers()["positions"], 8, n, idx).view(np.int64)[:, 0].astype(np.float64)}
+        for i, c in enumerate(wl.proj):
+            t, w = wl.descs[c]
+            raw = rows_of(*res.column_device(i), n, idx)
+            out[f"col{c}"] = (raw[:, :w].astype(np.float32) if t == N.ATTR_STRING else
+                              raw.view(np.int32)[:, 0].astype(np.float64) if t == N.ATTR_INTEGER else raw.view(np.float32)[:, 0])
+        aggs = []
+        for a, (kind, col) in enumerate(wl.aggs):
+            gi, gf, valid = res.agg(a)
+            integral = kind == N.AGG_COUNT or wl.descs[col][0] == N.ATTR_INTEGER
+            aggs.append((float(gi) if integral else gf) if valid else np.nan)
+        out["aggs"] = np.asarray(aggs, dtype=np.float64)
+        for name, arr in out.items():
+            np.save(os.path.join(out_dir, f"sel{s}_{name}.npy"), arr)
+
+
 def scan_host_rows(ctx, mbcol, wl, host_cols, rows, terms, want, position_base):
     """Context.scan_host with the row count given explicitly (untouched columns are passed as a dummy buffer)."""
     import ctypes as C
@@ -703,11 +754,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-pageable", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="tuning runs only: skip the end-to-end leg (the line then carries e2e: null)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as .npy files under DIR (one GPU)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl != "ours" or max(world, args.gpus) > 1):
+        ap.error("--dump-outputs writes the outputs of the GPU path on one GPU (--impl ours --gpus 1)")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
