@@ -201,6 +201,16 @@ int32_t mbc_bitmap_values(mbc_table* t, int32_t col, const void** values, int64_
 /* Columnarfile.java:1103-1127 getBitmapIndex(col,value).getBitSet(): copies the value's bitmap
  * into out_words (BitSet.toLongArray() order); all-zero when the value was never indexed. */
 int32_t mbc_bitmap_get(mbc_table* t, int32_t col, const void* value, uint64_t* out_words, int64_t nwords);
+/* Physical layout of a column's bitmap index, chosen by mbc_bitmap_build; every call above returns the same either way.
+ *   DENSE : one uncompressed bitset per distinct value, D * N/8 bytes of HBM.
+ *   SPARSE: the indexed row ids sorted by value (4 bytes per row) plus the N/8-byte bitmap of the rows the index
+ *           covers; taken when the column has more than 2^19 distinct values or its bitsets do not fit the device.
+ * Returns the MBC_BITMAP_* layout (NONE when the column has no index) and, when device_bytes is not NULL, the
+ * index's HBM bytes; < 0 on a bad argument. */
+#define MBC_BITMAP_NONE   0
+#define MBC_BITMAP_DENSE  1
+#define MBC_BITMAP_SPARSE 2
+int32_t mbc_bitmap_layout(const mbc_table* t, int32_t col, int64_t* device_bytes);
 
 /* ---- K4 (+K5): bitmap CNF scan ------------------------------------------------------- */
 /* Replaces index/ColumnarIndexScan.java:79-182,185-268 (CNF over per-term bitsets),

@@ -22,6 +22,7 @@ OPERAND_LITERAL, OPERAND_OUTER, OPERAND_INNER = 0, 1, 2
 WANT_POSITIONS, WANT_COLUMNS, WANT_TUPLES, WANT_AGG, WANT_BITMAP, WANT_HOST = 1, 2, 4, 8, 16, 32
 AGG_COUNT, AGG_SUM, AGG_MIN, AGG_MAX = 0, 1, 2, 3
 ERR_ARG, ERR_CUDA, ERR_NODEVICE, ERR_UNSUPPORTED, ERR_FORMAT, ERR_NOINDEX = -1, -2, -3, -4, -5, -6
+BITMAP_NONE, BITMAP_DENSE, BITMAP_SPARSE = 0, 1, 2
 
 
 class mbc_coldesc(C.Structure):
@@ -87,6 +88,7 @@ _SIGNATURES = {
     "mbc_bitmap_exists": (C.c_int32, [_VP, C.c_int32]),
     "mbc_bitmap_values": (C.c_int32, [_VP, C.c_int32, C.POINTER(_VP), C.POINTER(C.c_int64)]),
     "mbc_bitmap_get": (C.c_int32, [_VP, C.c_int32, _VP, _VP, C.c_int64]),
+    "mbc_bitmap_layout": (C.c_int32, [_VP, C.c_int32, C.POINTER(C.c_int64)]),
     "mbc_bitmap_scan": (C.c_int32, [_VP, C.POINTER(mbc_term), C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.c_uint32,
                                     C.POINTER(mbc_aggspec), C.c_int32, C.POINTER(_VP)]),
     "mbc_bitmap_join": (C.c_int32, [_VP, _VP, _VP, _VP, C.POINTER(mbc_term), C.c_int32, C.POINTER(mbc_projspec),

@@ -319,6 +319,8 @@ void mbc_table_free(mbc_table* t) {
     for (auto& b : t->bm) {
         dev_free(t->ctx, b.d_words);
         dev_free(t->ctx, b.d_ids);
+        dev_free(t->ctx, b.d_rows);
+        dev_free(t->ctx, b.d_indexed);
     }
     dev_free(t->ctx, t->d_deleted);
     mbc_ctx* ctx = t->ctx;

@@ -86,6 +86,14 @@ struct BitmapIndex {
     uint32_t* d_words = nullptr;
     int32_t   chunk_rows = 0;      // rows per chunk (power of two, 1024..8192)
     uint32_t* d_ids   = nullptr;   // per-row dense value id (kept for the join's low-cardinality path)
+    // sparse layout (value-sorted position lists), built where the per-value bitsets above cannot be (mbc_bitmap.cu):
+    // value v's rows are d_rows[offsets[v] .. offsets[v+1]), ascending.  The offsets stay on the host: every reader (the
+    // scan's binary search and row counts, mbc_bitmap_get) needs them there, and no kernel reads them.
+    bool      sparse = false;
+    uint32_t* d_rows = nullptr;    // n_indexed local row ids ordered by (value id, row)
+    uint32_t* d_indexed = nullptr; // words_pad words: the rows that were live when the index was built
+    int64_t   n_indexed = 0;
+    std::vector<uint32_t> offsets; // nvalues + 1
 };
 
 }  // namespace mbc
@@ -208,5 +216,17 @@ int32_t finish_result_host(mbc_result* r);     // tuple encode + D2H according t
 // stable LSD radix sort of (key, value) pairs by the low key_bits bits of the keys, in place (mbc_join.cu)
 // pass_mask: bit p = run the pass over key bits [8p, 8p+8) (clear it for digits known to be constant)
 int32_t radix_sort_pairs(mbc_ctx* ctx, uint32_t* d_keys, uint32_t* d_vals, int64_t n, int key_bits, uint32_t pass_mask = 0xFu);
+// exclusive scan of n uint32 counts into n+1 uint64 offsets, total in d_out[n] (mbc_join.cu)
+int32_t exclusive_scan_u32(mbc_ctx* ctx, const uint32_t* d_in, int64_t n, unsigned long long* d_out);
+
+// ---- row-id sorting shared by mbc_sort and the sparse bitmap layout (mbc_sort.cu) ---------------------------------
+// rows[i] = pos[i] - base
+__global__ void __launch_bounds__(256) sort_rows_from_positions_kernel(const int64_t* __restrict__ pos, int64_t n, int64_t base,
+                                                                      uint32_t* __restrict__ rows);
+// out row i = column row rows[i] (stride bytes, a multiple of 4)
+__global__ void __launch_bounds__(256) sort_gather_kernel(const uint32_t* __restrict__ rows, int64_t n, const void* src, int stride, void* dst);
+// stable reorder of the row ids `rows` by column c (every 32-bit word of its key, least significant first), so rows
+// with equal keys keep their order; keys (n words) and bits (2 words) are scratch
+int32_t sort_rows_by_column(mbc_ctx* ctx, uint32_t* rows, int64_t n, const Column& c, bool descending, uint32_t* keys, uint32_t* bits);
 
 }  // namespace mbc

@@ -124,7 +124,7 @@ __global__ void __launch_bounds__(kScanBlock) xscan_apply_kernel(const uint32_t*
     if (blockIdx.x == gridDim.x - 1 && threadIdx.x == kScanBlock - 1) out[n] = block_sums[gridDim.x];
 }
 
-static int32_t exclusive_scan_u32(mbc_ctx* ctx, const uint32_t* d_in, int64_t n, unsigned long long* d_out /* n+1 */) {
+int32_t exclusive_scan_u32(mbc_ctx* ctx, const uint32_t* d_in, int64_t n, unsigned long long* d_out /* n+1 */) {
     if (n == 0) {
         MBC_CUDA(cudaMemsetAsync(d_out, 0, 8, ctx->stream));
         return MBC_OK;

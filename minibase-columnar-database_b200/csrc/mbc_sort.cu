@@ -62,6 +62,28 @@ __global__ void __launch_bounds__(256) sort_gather_kernel(const uint32_t* __rest
     }
 }
 
+int32_t sort_rows_by_column(mbc_ctx* ctx, uint32_t* rows, int64_t n, const Column& c, bool descending, uint32_t* keys, uint32_t* bits) {
+    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, (int64_t)ctx->sm_count * 8));
+    const int words = c.type == MBC_ATTR_STRING ? (c.width + 3) / 4 : 1;      // bytes past the width are zero padding
+    for (int w = words - 1; w >= 0; --w) {
+        sort_key_kernel<<<grid, 256, 0, ctx->stream>>>(rows, n, c.d, c.stride, w, c.type, descending ? 1 : 0, keys);
+        // which of the four digits vary at all (small int domains, zero padding and common prefixes of strings do not)
+        const uint32_t preset[2] = {0u, ~0u};
+        uint32_t seen[2];
+        MBC_CUDA(cudaMemcpyAsync(bits, preset, 8, cudaMemcpyHostToDevice, ctx->stream));
+        sort_key_bits_kernel<<<grid, 256, 0, ctx->stream>>>(keys, n, bits);
+        ctx->launches += 2;
+        MBC_CUDA(cudaMemcpyAsync(seen, bits, 8, cudaMemcpyDeviceToHost, ctx->stream));
+        MBC_CUDA(cudaStreamSynchronize(ctx->stream));
+        const uint32_t differ = seen[0] ^ seen[1];
+        uint32_t pass_mask = 0;
+        for (int b = 0; b < 4; ++b)
+            if ((differ >> (8 * b)) & 0xFFu) pass_mask |= 1u << b;
+        MBC_TRY(radix_sort_pairs(ctx, keys, rows, n, 32, pass_mask));
+    }
+    return MBC_OK;
+}
+
 }  // namespace mbc
 
 using namespace mbc;
@@ -112,26 +134,7 @@ extern "C" int32_t mbc_sort(mbc_table* t, const int32_t* key_cols, int32_t nkeys
         STRY(dev_alloc(ctx, (void**)&bits, 8, false));
         sort_rows_from_positions_kernel<<<grid, 256, 0, ctx->stream>>>(all->d_pos, n, t->pos_base, rows);
         ctx->launches++;
-        for (int k = nkeys - 1; k >= 0; --k) {
-            const Column& c = t->cols[key_cols[k]];
-            const int words = c.type == MBC_ATTR_STRING ? (c.width + 3) / 4 : 1;      // bytes past the width are zero padding
-            for (int w = words - 1; w >= 0; --w) {
-                sort_key_kernel<<<grid, 256, 0, ctx->stream>>>(rows, n, c.d, c.stride, w, c.type, descending ? 1 : 0, keys);
-                // which of the four digits vary at all (small int domains, zero padding and common prefixes of strings do not)
-                const uint32_t preset[2] = {0u, ~0u};
-                uint32_t seen[2];
-                if (cudaMemcpyAsync(bits, preset, 8, cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess) return fail(MBC_ERR_CUDA);
-                sort_key_bits_kernel<<<grid, 256, 0, ctx->stream>>>(keys, n, bits);
-                ctx->launches += 2;
-                if (cudaMemcpyAsync(seen, bits, 8, cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess ||
-                    cudaStreamSynchronize(ctx->stream) != cudaSuccess) return fail(MBC_ERR_CUDA);
-                const uint32_t differ = seen[0] ^ seen[1];
-                uint32_t pass_mask = 0;
-                for (int b = 0; b < 4; ++b)
-                    if ((differ >> (8 * b)) & 0xFFu) pass_mask |= 1u << b;
-                STRY(radix_sort_pairs(ctx, keys, rows, n, 32, pass_mask));
-            }
-        }
+        for (int k = nkeys - 1; k >= 0; --k) STRY(sort_rows_by_column(ctx, rows, n, t->cols[key_cols[k]], descending != 0, keys, bits));
     }
     if ((want & MBC_WANT_POSITIONS) && n > 0) {
         STRY(dev_alloc(ctx, (void**)&r->d_pos, (size_t)n * 8, false));

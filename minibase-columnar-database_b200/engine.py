@@ -247,6 +247,14 @@ class Table:
     def bitmap_exists(self, col: int) -> bool:
         return bool(N.lib().mbc_bitmap_exists(self._h, col))
 
+    def bitmap_layout(self, col: int) -> tuple[int, int]:
+        """(BITMAP_NONE / BITMAP_DENSE / BITMAP_SPARSE, HBM bytes) of the column's bitmap index."""
+        nbytes = C.c_int64()
+        layout = N.lib().mbc_bitmap_layout(self._h, col, C.byref(nbytes))
+        if layout < 0:
+            N.check(layout)
+        return int(layout), int(nbytes.value)
+
     def bitmap_values(self, col: int):
         p, n = C.c_void_p(), C.c_int64()
         N.check(N.lib().mbc_bitmap_values(self._h, col, C.byref(p), C.byref(n)))
