@@ -236,7 +236,8 @@ int32_t mbc_bitmap_join(mbc_table* outer, mbc_table* inner,
 
 /* ---- sort (input/ColumnarSort.java:73-400: `sort DB CF [sort columns] [projection] ASC|DSC ...`) --------------
  * Rows ordered by the key columns, first key most significant: ints numerically, strings in byte order
- * (= String.compareTo for BMP text, the comparator of ColumnarSort.java:163-205), reals numerically; `descending`
+ * (= String.compareTo for BMP text, the comparator of ColumnarSort.java:163-205), reals numerically (-0.0 and +0.0
+ * are equal keys; NaN is not a supported key value); `descending`
  * reverses all keys at once.  Equal keys come out in ascending position (the reference's external merge leaves the
  * order of ties unspecified).  Deleted rows are skipped.  The result carries the positions in sorted order
  * (MBC_WANT_POSITIONS) and the projected columns / Tuple bytes of those rows (MBC_WANT_COLUMNS / MBC_WANT_TUPLES). */

@@ -12,14 +12,18 @@
 
 namespace mbc {
 
-// key word of every row id in `rows`: ints biased to unsigned order, reals mapped to their total order, string words
-// byte-swapped so that unsigned compare = byte order; complemented for a descending sort
+// key word of every row id in `rows`: ints biased to unsigned order, reals mapped to their total order (with -0.0 taken
+// as +0.0 first: the reference compares reals with float ==, so the two zeros are one key and tie by position), string
+// words byte-swapped so that unsigned compare = byte order; complemented for a descending sort
 __global__ void __launch_bounds__(256) sort_key_kernel(const uint32_t* __restrict__ rows, int64_t n, const void* col, int stride, int word,
                                                        int type, int descending, uint32_t* __restrict__ keys) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         uint32_t v = reinterpret_cast<const uint32_t*>(reinterpret_cast<const char*>(col) + (size_t)rows[i] * stride)[word];
         if (type == MBC_ATTR_INTEGER) v ^= 0x80000000u;
-        else if (type == MBC_ATTR_REAL) v = (v & 0x80000000u) ? ~v : (v | 0x80000000u);
+        else if (type == MBC_ATTR_REAL) {
+            if (v == 0x80000000u) v = 0u;
+            v = (v & 0x80000000u) ? ~v : (v | 0x80000000u);
+        }
         else v = __byte_perm(v, 0, 0x0123);
         keys[i] = descending ? ~v : v;
     }
