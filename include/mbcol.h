@@ -313,8 +313,10 @@ const void*    mbc_result_column(const mbc_result* r, int32_t i, int32_t* width)
 /* reference Tuple byte layout, big-endian: [fldCnt:2][fldOffset[0..n]:2 each][fields],
  * strings as [len:2][modified UTF-8][zero pad] (heap/Tuple.java:369-440). */
 const uint8_t* mbc_result_tuples(const mbc_result* r, int32_t* tuple_len);
-/* aggregate i: valid=0 for MIN/MAX over an empty set. Integer aggregates are exact in as_i64;
- * real SUM is a double sum, MIN/MAX of reals are exact floats widened to double. */
+/* aggregate i: valid=0 for MIN/MAX over an empty set. Integer aggregates are exact in as_i64; a real aggregate's as_i64
+ * is Java's (long) of its double: truncated toward zero, INT64_MIN / INT64_MAX when out of range (±inf included), 0 for NaN.
+ * Real SUM is a double sum, MIN/MAX of reals are exact floats widened to double (the sign of a MIN/MAX that is a zero is
+ * not specified when the set holds both -0.0 and +0.0; NaN inputs are outside the contract). */
 int32_t        mbc_result_agg(const mbc_result* r, int32_t i, int64_t* as_i64, double* as_f64, int32_t* valid);
 /* qualifying set as BitSet.toLongArray() words (needs MBC_WANT_BITMAP|MBC_WANT_HOST) */
 const uint64_t* mbc_result_bitmap(const mbc_result* r, int64_t* nwords);

@@ -146,7 +146,7 @@ int32_t result_finalize(mbc_result* r) {
             double d;
             memcpy(&d, &r->h_small[a], 8);
             g.f = d;
-            g.i = (int64_t)d;
+            g.i = real_agg_as_i64(d);
         }
         g.valid = (g.kind == MBC_AGG_COUNT || g.kind == MBC_AGG_SUM) ? 1 : (r->count > 0);
         if (!g.valid) { g.i = 0; g.f = 0.0; }

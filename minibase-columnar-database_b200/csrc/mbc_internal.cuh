@@ -37,6 +37,15 @@ constexpr int kMaxStrStride = 256; // widest device string row
 
 static inline int64_t round_up(int64_t x, int64_t m) { return (x + m - 1) / m * m; }
 
+// as_i64 of a real aggregate, with Java's (long) d semantics: truncated toward zero, saturated to INT64_MIN / INT64_MAX
+// out of range (±inf included), 0 for NaN.  A plain (int64_t) cast of such a double (MAX over FLT_MAX) is undefined.
+static inline int64_t real_agg_as_i64(double d) {
+    if (d != d) return 0;
+    if (d >= 9223372036854775808.0) return INT64_MAX;    // 2^63
+    if (d < -9223372036854775808.0) return INT64_MIN;
+    return (int64_t)d;
+}
+
 // device row stride of a char(width) column: multiples of 4 below 16, multiples of 16 above,
 // so every row is reachable with aligned 32-bit or 128-bit loads.  Padding bytes are zero.
 static inline int str_stride(int width) {

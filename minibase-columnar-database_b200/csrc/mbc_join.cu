@@ -1308,7 +1308,7 @@ extern "C" int32_t mbc_bitmap_join(mbc_table* outer, mbc_table* inner, const mbc
             g.type = ja[a].type;
             const bool integral = g.kind == MBC_AGG_COUNT || g.type == MBC_ATTR_INTEGER;
             if (integral) { g.i = (int64_t)agg_raw[a]; g.f = (double)g.i; }
-            else { double d; memcpy(&d, &agg_raw[a], 8); g.f = d; g.i = (int64_t)d; }
+            else { double d; memcpy(&d, &agg_raw[a], 8); g.f = d; g.i = real_agg_as_i64(d); }
             g.valid = (g.kind == MBC_AGG_COUNT || g.kind == MBC_AGG_SUM) ? 1 : (npairs > 0);
             if (!g.valid) { g.i = 0; g.f = 0.0; }
         }

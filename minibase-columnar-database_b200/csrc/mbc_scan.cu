@@ -226,7 +226,7 @@ void decode_aggs(mbc_result* r, const DevAgg* dev, int nagg, const unsigned long
             double d;
             memcpy(&d, &raw[a], 8);
             g.f = d;
-            g.i = (int64_t)d;
+            g.i = real_agg_as_i64(d);
         }
         g.valid = (g.kind == MBC_AGG_COUNT || g.kind == MBC_AGG_SUM) ? 1 : (r->count > 0);
         if (!g.valid) { g.i = 0; g.f = 0.0; }

@@ -503,7 +503,7 @@ int32_t mbc_shard_agg(const mbc_shard* s, int32_t i, int32_t kind, int32_t type,
         else { ai = std::max(ai, vi); af = std::max(af, vf); }
     }
     const bool ok = !first && (kind == MBC_AGG_COUNT || kind == MBC_AGG_SUM || s->total > 0);
-    if (as_i64) *as_i64 = ok ? (integral ? ai : (long long)af) : 0;
+    if (as_i64) *as_i64 = ok ? (integral ? ai : real_agg_as_i64(af)) : 0;
     if (as_f64) *as_f64 = ok ? (integral ? (double)ai : af) : 0.0;
     if (valid) *valid = ok ? 1 : 0;
     return MBC_OK;

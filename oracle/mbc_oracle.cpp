@@ -239,6 +239,14 @@ inline void project_field(const TupleDesc& sd, const uint8_t* src, int src_col, 
     }
 }
 
+// as_i64 of a real aggregate: Java's (long) d -- toward zero, saturated to INT64_MIN / INT64_MAX (±inf too), NaN -> 0
+inline int64_t real_as_i64(double d) {
+    if (d != d) return 0;
+    if (d >= 9223372036854775808.0) return INT64_MAX;
+    if (d < -9223372036854775808.0) return INT64_MIN;
+    return (int64_t)d;
+}
+
 struct AggState {
     int kind, type;
     int64_t i = 0;
@@ -271,7 +279,7 @@ struct AggState {
         bool integral = kind == AGG_COUNT || type == ATTR_INTEGER;
         bool valid = kind == AGG_COUNT || kind == AGG_SUM || any;
         o->valid = valid;
-        o->i = valid ? (integral ? i : (int64_t)f) : 0;
+        o->i = valid ? (integral ? i : real_as_i64(f)) : 0;
         o->f = valid ? (integral ? (double)i : f) : 0.0;
     }
 };

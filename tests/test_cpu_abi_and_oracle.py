@@ -173,6 +173,32 @@ def test_two_strategies_agree_on_random_tables(oracle):
             np.testing.assert_array_equal(oracle.positions_from_bits(bits, n), rows["positions"])
 
 
+def test_real_aggregate_as_i64_is_javas_long_cast(oracle):
+    """as_i64 of a real aggregate is Java's (long) d: toward zero, saturated out of range (±inf too), NaN -> 0 -- where a
+    plain C cast of MAX over FLT_MAX is undefined behaviour."""
+    fmax = float(np.finfo(np.float32).max)
+    r = np.array([1.5, fmax, np.inf, -2.75, -fmax, 0.0], dtype=np.float32)
+    descs = [(2, 4), (1, 4)]
+    cols = [r, np.arange(r.size, dtype=np.int32)]
+    aggs = [(3, 0), (2, 0), (1, 0)]                                  # MAX, MIN, SUM
+    cases = [(None, [(2**63 - 1, np.inf), (-2**63, -fmax), (2**63 - 1, np.inf)]),    # all rows
+             ([oracle.Term(oracle.OP_EQ, ("col", 1), ("int", 1), 0)],              # FLT_MAX alone: out of range, finite
+              [(2**63 - 1, fmax), (2**63 - 1, fmax), (2**63 - 1, fmax)]),
+             ([oracle.Term(oracle.OP_GE, ("col", 1), ("int", 3), 0), oracle.Term(oracle.OP_LT, ("col", 1), ("int", 4), 1)],
+              [(-2, -2.75), (-2, -2.75), (-2, -2.75)]),                             # truncation toward zero
+             ([oracle.Term(oracle.OP_GE, ("col", 1), ("int", 4), 0)],
+              [(0, 0.0), (-2**63, -fmax), (-2**63, -fmax)])]
+    for terms, want in cases:
+        got = oracle.scan(descs, cols, terms or [], aggs=aggs)["aggs"]
+        assert [(i, f) for i, f, _ in got] == want, (terms, got)
+    # +inf + -inf is NaN, whose integer view is 0
+    both = np.array([np.inf, -np.inf], dtype=np.float32)
+    i, f, v = oracle.scan([(2, 4)], [both], [], aggs=[(1, 0)])["aggs"][0]
+    assert v and np.isnan(f) and i == 0
+    i, f, v = oracle.scan([(2, 4)], [both], [], aggs=[(3, 0)])["aggs"][0]
+    assert v and f == np.inf and i == 2**63 - 1
+
+
 def test_oracle_threads_agree(oracle):
     n = 200_003
     descs = [(1, 4), (2, 4), (0, 16)]
