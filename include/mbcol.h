@@ -244,6 +244,22 @@ int32_t mbc_bitmap_join(mbc_table* outer, mbc_table* inner,
 int32_t mbc_sort(mbc_table* t, const int32_t* key_cols, int32_t nkeys, int32_t descending,
                  const int32_t* proj_cols, int32_t nproj, uint32_t want, mbc_result** out);
 
+/* ---- grouped aggregation (absent from the reference, like the aggregates of SURVEY.md 8c) ------------------------
+ * GROUP BY key_cols over the rows of t that satisfy the CNF (same term rules as mbc_scan; nterms == 0 = every row),
+ * deleted rows skipped.  One output row per distinct key tuple, groups in ascending key order (first key most
+ * significant; ints numerically, strings in byte order, reals numerically: the order of mbc_sort ascending).
+ * -0.0 and +0.0 are one key.  NaN keys are outside the contract.
+ *   MBC_WANT_COLUMNS   : the key values of each group, as result column k for key k (mbc_result_column);
+ *                        the values are those of the group's lowest-position row
+ *   MBC_WANT_POSITIONS : the lowest qualifying position of each group
+ *   MBC_WANT_AGG       : aggregates[i] per group (mbc_result_group_agg)
+ *   MBC_WANT_HOST      : copy what was asked for to the host
+ * mbc_result_count = number of groups.  MBC_WANT_TUPLES / MBC_WANT_BITMAP: MBC_ERR_UNSUPPORTED.
+ * Limits as mbc_sort / mbc_scan: <= 16 key columns, <= 8 aggregates, <= 2^32 rows in the table. */
+int32_t mbc_group_aggregate(mbc_table* t, const mbc_term* terms, int32_t nterms,
+                            const int32_t* key_cols, int32_t nkeys,
+                            const mbc_aggspec* aggs, int32_t nagg, uint32_t want, mbc_result** out);
+
 /* ---- sharding: TID-range shards on the GPUs of one node (SURVEY.md 8e) ----------------------------------------
  * The reference has no partitioning (it is one Java thread); this is what running its ColumnarFileScan
  * (iterator/ColumnarFileScan.java:156-188) over a table whose position ranges live on several GPUs needs: every rank
@@ -318,6 +334,11 @@ const uint8_t* mbc_result_tuples(const mbc_result* r, int32_t* tuple_len);
  * Real SUM is a double sum, MIN/MAX of reals are exact floats widened to double (the sign of a MIN/MAX that is a zero is
  * not specified when the set holds both -0.0 and +0.0; NaN inputs are outside the contract). */
 int32_t        mbc_result_agg(const mbc_result* r, int32_t i, int64_t* as_i64, double* as_f64, int32_t* valid);
+/* aggregate i of a grouped result, one entry per group (host; needs MBC_WANT_AGG | MBC_WANT_HOST).  Entry g is the pair
+ * mbc_result_agg would return for that aggregate over group g's rows (every group is non-empty, so always valid).
+ * The arrays stay owned by the result.  Calling mbc_result_agg on a grouped result, or this on any other result,
+ * returns MBC_ERR_ARG. */
+int32_t        mbc_result_group_agg(const mbc_result* r, int32_t i, const int64_t** as_i64, const double** as_f64);
 /* qualifying set as BitSet.toLongArray() words (needs MBC_WANT_BITMAP|MBC_WANT_HOST) */
 const uint64_t* mbc_result_bitmap(const mbc_result* r, int64_t* nwords);
 /* device-resident views (always available for what was asked): for NCCL gathers */

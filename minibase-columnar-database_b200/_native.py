@@ -94,6 +94,8 @@ _SIGNATURES = {
     "mbc_bitmap_join": (C.c_int32, [_VP, _VP, _VP, _VP, C.POINTER(mbc_term), C.c_int32, C.POINTER(mbc_projspec),
                                     C.c_int32, C.c_uint32, C.POINTER(mbc_aggspec), C.c_int32, C.POINTER(_VP)]),
     "mbc_sort": (C.c_int32, [_VP, C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.c_uint32, C.POINTER(_VP)]),
+    "mbc_group_aggregate": (C.c_int32, [_VP, C.POINTER(mbc_term), C.c_int32, C.POINTER(C.c_int32), C.c_int32,
+                                        C.POINTER(mbc_aggspec), C.c_int32, C.c_uint32, C.POINTER(_VP)]),
     "mbc_result_count": (C.c_int64, [_VP]),
     "mbc_result_kernel_ms": (C.c_float, [_VP]),
     "mbc_result_phase_ms": (C.c_int32, [_VP, C.POINTER(C.c_float)]),
@@ -102,6 +104,7 @@ _SIGNATURES = {
     "mbc_result_column": (_VP, [_VP, C.c_int32, C.POINTER(C.c_int32)]),
     "mbc_result_tuples": (_VP, [_VP, C.POINTER(C.c_int32)]),
     "mbc_result_agg": (C.c_int32, [_VP, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_double), C.POINTER(C.c_int32)]),
+    "mbc_result_group_agg": (C.c_int32, [_VP, C.c_int32, C.POINTER(_VP), C.POINTER(_VP)]),
     "mbc_result_bitmap": (_VP, [_VP, C.POINTER(C.c_int64)]),
     "mbc_result_device": (C.c_int32, [_VP, C.POINTER(_VP), C.POINTER(_VP), C.POINTER(_VP), C.POINTER(_VP)]),
     "mbc_result_column_device": (C.c_int32, [_VP, C.c_int32, C.POINTER(_VP), C.POINTER(C.c_int32)]),

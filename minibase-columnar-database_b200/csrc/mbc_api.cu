@@ -138,22 +138,25 @@ int32_t result_finalize(mbc_result* r) {
     r->count = (int64_t)r->h_small[kMaxAgg];
     for (size_t a = 0; a < r->aggs.size(); ++a) {
         mbc_result::Agg& g = r->aggs[a];
-        const bool integral = g.kind == MBC_AGG_COUNT || g.type == MBC_ATTR_INTEGER;
-        if (integral) {
-            g.i = (int64_t)r->h_small[a];
-            g.f = (double)g.i;
-        } else {
-            double d;
-            memcpy(&d, &r->h_small[a], 8);
-            g.f = d;
-            g.i = real_agg_as_i64(d);
-        }
-        g.valid = (g.kind == MBC_AGG_COUNT || g.kind == MBC_AGG_SUM) ? 1 : (r->count > 0);
-        if (!g.valid) { g.i = 0; g.f = 0.0; }
+        agg_from_raw(g.kind, g.type, r->h_small[a], r->count > 0, &g.i, &g.f, &g.valid);
     }
     if (r->ev_t0 && r->ev_t1 && cudaEventElapsedTime(&r->kernel_ms, r->ev_t0, r->ev_t1) != cudaSuccess) r->kernel_ms = -1.f;
     result_phase_times(r);
     return MBC_OK;
+}
+
+void agg_from_raw(int32_t kind, int32_t type, unsigned long long raw, bool nonempty, int64_t* i, double* f, int32_t* valid) {
+    if (kind == MBC_AGG_COUNT || type == MBC_ATTR_INTEGER) {
+        *i = (int64_t)raw;
+        *f = (double)*i;
+    } else {
+        double d;
+        memcpy(&d, &raw, 8);
+        *f = d;
+        *i = real_agg_as_i64(d);
+    }
+    *valid = (kind == MBC_AGG_COUNT || kind == MBC_AGG_SUM) ? 1 : nonempty;
+    if (!*valid) { *i = 0; *f = 0.0; }
 }
 
 void split_timing(mbc_ctx* ctx) {
@@ -433,12 +436,23 @@ const uint8_t* mbc_result_tuples(const mbc_result* r, int32_t* tuple_len) {
 }
 
 int32_t mbc_result_agg(const mbc_result* r, int32_t i, int64_t* as_i64, double* as_f64, int32_t* valid) {
+    if (r && r->grouped) MBC_FAIL(MBC_ERR_ARG, "mbc_result_agg: a grouped result has one value per group (mbc_result_group_agg)");
     if (!r || i < 0 || i >= (int)r->aggs.size()) MBC_FAIL(MBC_ERR_ARG, "mbc_result_agg: index %d of %d", i,
                                                           r ? (int)r->aggs.size() : 0);
     MBC_TRY(result_finalize(const_cast<mbc_result*>(r)));
     if (as_i64) *as_i64 = r->aggs[i].i;
     if (as_f64) *as_f64 = r->aggs[i].f;
     if (valid) *valid = r->aggs[i].valid;
+    return MBC_OK;
+}
+
+int32_t mbc_result_group_agg(const mbc_result* r, int32_t i, const int64_t** as_i64, const double** as_f64) {
+    if (!r || !r->grouped) MBC_FAIL(MBC_ERR_ARG, "mbc_result_group_agg: not a result of mbc_group_aggregate");
+    if (i < 0 || i >= (int)r->group_aggs.size())
+        MBC_FAIL(MBC_ERR_ARG, "mbc_result_group_agg: index %d of %d aggregates on the host (MBC_WANT_AGG | MBC_WANT_HOST)", i,
+                 (int)r->group_aggs.size());
+    if (as_i64) *as_i64 = r->group_aggs[i].i.data();
+    if (as_f64) *as_f64 = r->group_aggs[i].f.data();
     return MBC_OK;
 }
 

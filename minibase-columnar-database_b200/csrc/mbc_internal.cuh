@@ -177,6 +177,10 @@ struct mbc_result {
     // aggregates
     struct Agg { int32_t kind, type; int64_t i; double f; int32_t valid; };
     std::vector<Agg> aggs;
+    // mbc_group_aggregate: one row per group; d_aggs holds nagg x count raw values, group_aggs their host decode
+    bool grouped = false;
+    struct GroupAgg { std::vector<int64_t> i; std::vector<double> f; };
+    std::vector<GroupAgg> group_aggs;
     // Deferred completion (device-resident results of mbc_scan): the call returns with its kernels and the small
     // count/aggregate copy queued; the first accessor that needs the count waits on ev_ready.  Back-to-back scans
     // then run without host gaps between them.
@@ -205,6 +209,9 @@ void    split_timing(mbc_ctx* ctx);
 void    result_phase_times(mbc_result* r);  // fills phase_ms from the events of a completed resident scan
 int32_t result_finalize(mbc_result* r);   // wait for a deferred result's count/aggregates (no-op when final)
 cudaEvent_t event_get(mbc_ctx* ctx);
+// one aggregate from its raw 8 bytes (int64 for COUNT and integer columns, else the bits of a double): exact integers, a
+// real's as_i64 through real_agg_as_i64; MIN / MAX over an empty set are invalid and read 0
+void    agg_from_raw(int32_t kind, int32_t type, unsigned long long raw, bool nonempty, int64_t* i, double* f, int32_t* valid);
 void    event_put(mbc_ctx* ctx, cudaEvent_t e);        // close a timed segment (sync), keep its time, the next begin_timing adds to it
 
 // ---- the select -> compact -> project -> aggregate engine (mbc_scan.cu) ---------------------
@@ -234,6 +241,12 @@ __global__ void __launch_bounds__(256) sort_rows_from_positions_kernel(const int
                                                                       uint32_t* __restrict__ rows);
 // out row i = column row rows[i] (stride bytes, a multiple of 4)
 __global__ void __launch_bounds__(256) sort_gather_kernel(const uint32_t* __restrict__ rows, int64_t n, const void* src, int stride, void* dst);
+// pos[i] = base + rows[i]
+__global__ void __launch_bounds__(256) sort_positions_kernel(const uint32_t* __restrict__ rows, int64_t n, int64_t base, int64_t* __restrict__ pos);
+// run d = run_of[i] of a head i starts at element i: start[d] = i, head_row[d] = rows[i] (mbc_bitmap.cu)
+__global__ void __launch_bounds__(256) sparse_run_starts_kernel(const uint32_t* __restrict__ head, const unsigned long long* __restrict__ run_of,
+                                                                const uint32_t* __restrict__ rows, int64_t n, uint32_t* __restrict__ start,
+                                                                uint32_t* __restrict__ head_row);
 // stable reorder of the row ids `rows` by column c (every 32-bit word of its key, least significant first), so rows
 // with equal keys keep their order; keys (n words) and bits (2 words) are scratch
 int32_t sort_rows_by_column(mbc_ctx* ctx, uint32_t* rows, int64_t n, const Column& c, bool descending, uint32_t* keys, uint32_t* bits);

@@ -218,18 +218,7 @@ void decode_aggs(mbc_result* r, const DevAgg* dev, int nagg, const unsigned long
         mbc_result::Agg& g = r->aggs[a];
         g.kind = dev[a].kind;
         g.type = dev[a].type;
-        bool integral = g.kind == MBC_AGG_COUNT || g.type == MBC_ATTR_INTEGER;
-        if (integral) {
-            g.i = (int64_t)raw[a];
-            g.f = (double)g.i;
-        } else {
-            double d;
-            memcpy(&d, &raw[a], 8);
-            g.f = d;
-            g.i = real_agg_as_i64(d);
-        }
-        g.valid = (g.kind == MBC_AGG_COUNT || g.kind == MBC_AGG_SUM) ? 1 : (r->count > 0);
-        if (!g.valid) { g.i = 0; g.f = 0.0; }
+        agg_from_raw(g.kind, g.type, raw[a], r->count > 0, &g.i, &g.f, &g.valid);
     }
 }
 

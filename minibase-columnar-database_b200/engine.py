@@ -240,6 +240,19 @@ class Table:
         N.check(N.lib().mbc_sort(self._h, karr, len(key_cols), 1 if descending else 0, parr, len(proj), want, C.byref(h)))
         return Result(self.ctx, h, [self.coldescs[c] for c in proj], want, 0)
 
+    def group_aggregate(self, terms: Sequence[Term], key_cols: Sequence[int], aggs: Sequence[tuple] = (),
+                        want: int = N.WANT_COLUMNS | N.WANT_POSITIONS | N.WANT_AGG | N.WANT_HOST) -> "Result":
+        """GROUP BY key_cols over the rows that satisfy the CNF: one row per group in ascending key order.  The result's
+        columns are the key columns (values of each group's lowest-position row), its positions those rows' positions,
+        and group_agg(i) aggregate i of every group; count = number of groups."""
+        tarr, nt, keep = pack_terms(terms)
+        karr = (C.c_int32 * max(len(key_cols), 1))(*key_cols)
+        aarr = (N.mbc_aggspec * max(len(aggs), 1))(*[N.mbc_aggspec(int(k), int(c)) for k, c in aggs])
+        h = C.c_void_p()
+        N.check(N.lib().mbc_group_aggregate(self._h, tarr, nt, karr, len(key_cols), aarr, len(aggs), want, C.byref(h)))
+        del keep
+        return Result(self.ctx, h, [self.coldescs[c] for c in key_cols], want, len(aggs))
+
     # ---- bitmap indexes --------------------------------------------------------------------
     def bitmap_build(self, col: int) -> None:
         N.check(N.lib().mbc_bitmap_build(self._h, col))
@@ -354,6 +367,13 @@ class Result:
         a, f, v = C.c_int64(), C.c_double(), C.c_int32()
         N.check(N.lib().mbc_result_agg(self._h, i, C.byref(a), C.byref(f), C.byref(v)))
         return int(a.value), float(f.value), bool(v.value)
+
+    def group_agg(self, i: int) -> tuple:
+        """Aggregate i of a grouped result, one entry per group: (int64 array, float64 array), copies."""
+        a, f = C.c_void_p(), C.c_void_p()
+        N.check(N.lib().mbc_result_group_agg(self._h, i, C.byref(a), C.byref(f)))
+        n = self.count
+        return _np_from_ptr(a.value, n * 8, np.int64).copy(), _np_from_ptr(f.value, n * 8, np.float64).copy()
 
     def bitmap(self) -> np.ndarray:
         n = C.c_int64()

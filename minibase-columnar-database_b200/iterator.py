@@ -300,6 +300,28 @@ class ColumnarFileScan(Iterator):
         res.close()
         return out
 
+    def group_aggregate(self, key_fields: Sequence[int], specs: Sequence[tuple]) -> list:
+        """GROUP BY the 0-based columns key_fields over the rows OutputFilter selects; specs as in aggregate().  Returns
+        one (key values..., aggregate values...) tuple per group, groups in ascending key order: ints and COUNT / integer
+        aggregates as int, reals as float, strings as str."""
+        res = self.f.table.group_aggregate(flatten_condexpr(self.OutputFilter), list(key_fields), aggs=specs)
+        try:
+            keys = []
+            for k, col in enumerate(key_fields):
+                vals = res.column(k)
+                if self.f.attrTypes[col].attrType == AttrType.attrString:
+                    keys.append([bytes(r).split(b"\0", 1)[0].decode("utf-8") for r in vals])
+                else:
+                    keys.append(vals.tolist())
+            aggs = []
+            for a, (kind, col) in enumerate(specs):
+                i, f = res.group_agg(a)
+                integral = kind == N.AGG_COUNT or self.f.attrTypes[col].attrType == AttrType.attrInteger
+                aggs.append(i.tolist() if integral else f.tolist())
+            return [tuple(k[g] for k in keys) + tuple(a[g] for a in aggs) for g in range(res.count)]
+        finally:
+            res.close()
+
 
 class _ColumnsScan(Iterator):
     """Shared body of ColumnarColumnScan / ColumnarColumnsScan (SURVEY.md 8f rank 1): the predicate is evaluated over a
