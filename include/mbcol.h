@@ -244,6 +244,18 @@ int32_t mbc_bitmap_join(mbc_table* outer, mbc_table* inner,
 int32_t mbc_sort(mbc_table* t, const int32_t* key_cols, int32_t nkeys, int32_t descending,
                  const int32_t* proj_cols, int32_t nproj, uint32_t want, mbc_result** out);
 
+/* ---- top-k (ORDER BY ... LIMIT k; absent from the reference) ---------------------------------------------------------
+ * ORDER BY key_cols LIMIT k over the rows of t that satisfy the CNF (same term rules as mbc_scan; nterms == 0 = every row),
+ * deleted rows skipped.  The result is exactly the first min(k, Q) rows of mbc_sort's order over the Q qualifying rows:
+ * same keys, same direction, same tie order (equal keys in ascending position, in both directions), -0.0 and +0.0 one key.
+ * With k >= Q it is a filtered sort.
+ *   MBC_WANT_POSITIONS / MBC_WANT_COLUMNS / MBC_WANT_TUPLES / MBC_WANT_HOST as mbc_sort.
+ *   MBC_WANT_AGG / MBC_WANT_BITMAP: MBC_ERR_UNSUPPORTED.   k < 0: MBC_ERR_ARG.   k == 0: an empty result.
+ * Limits as mbc_sort: <= 16 key columns, <= 16 projected fields, <= 2^32 rows in the table. */
+int32_t mbc_topk(mbc_table* t, const mbc_term* terms, int32_t nterms,
+                 const int32_t* key_cols, int32_t nkeys, int32_t descending, int64_t k,
+                 const int32_t* proj_cols, int32_t nproj, uint32_t want, mbc_result** out);
+
 /* ---- grouped aggregation (absent from the reference, like the aggregates of SURVEY.md 8c) ------------------------
  * GROUP BY key_cols over the rows of t that satisfy the CNF (same term rules as mbc_scan; nterms == 0 = every row),
  * deleted rows skipped.  One output row per distinct key tuple, groups in ascending key order (first key most

@@ -96,6 +96,8 @@ _SIGNATURES = {
     "mbc_sort": (C.c_int32, [_VP, C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.c_uint32, C.POINTER(_VP)]),
     "mbc_group_aggregate": (C.c_int32, [_VP, C.POINTER(mbc_term), C.c_int32, C.POINTER(C.c_int32), C.c_int32,
                                         C.POINTER(mbc_aggspec), C.c_int32, C.c_uint32, C.POINTER(_VP)]),
+    "mbc_topk": (C.c_int32, [_VP, C.POINTER(mbc_term), C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.c_int64,
+                             C.POINTER(C.c_int32), C.c_int32, C.c_uint32, C.POINTER(_VP)]),
     "mbc_result_count": (C.c_int64, [_VP]),
     "mbc_result_kernel_ms": (C.c_float, [_VP]),
     "mbc_result_phase_ms": (C.c_int32, [_VP, C.POINTER(C.c_float)]),

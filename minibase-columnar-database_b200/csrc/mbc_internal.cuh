@@ -235,7 +235,13 @@ int32_t radix_sort_pairs(mbc_ctx* ctx, uint32_t* d_keys, uint32_t* d_vals, int64
 // exclusive scan of n uint32 counts into n+1 uint64 offsets, total in d_out[n] (mbc_join.cu)
 int32_t exclusive_scan_u32(mbc_ctx* ctx, const uint32_t* d_in, int64_t n, unsigned long long* d_out);
 
-// ---- row-id sorting shared by mbc_sort and the sparse bitmap layout (mbc_sort.cu) ---------------------------------
+// ---- row-id sorting shared by mbc_sort, the sparse bitmap layout and mbc_topk (mbc_sort.cu) ------------------------
+// keys[i] = 32-bit word `word` of column row rows[i] as an unsigned key in sort order (ints biased, reals in total order
+// with -0.0 as +0.0, string words byte-swapped), complemented when descending
+__global__ void __launch_bounds__(256) sort_key_kernel(const uint32_t* __restrict__ rows, int64_t n, const void* col, int stride, int word,
+                                                       int type, int descending, uint32_t* __restrict__ keys);
+// or_and[0] |= every key, or_and[1] &= every key (preset {0, ~0}): the digits where they agree are constant
+__global__ void __launch_bounds__(256) sort_key_bits_kernel(const uint32_t* __restrict__ keys, int64_t n, uint32_t* or_and);
 // rows[i] = pos[i] - base
 __global__ void __launch_bounds__(256) sort_rows_from_positions_kernel(const int64_t* __restrict__ pos, int64_t n, int64_t base,
                                                                       uint32_t* __restrict__ rows);

@@ -253,6 +253,19 @@ class Table:
         del keep
         return Result(self.ctx, h, [self.coldescs[c] for c in key_cols], want, len(aggs))
 
+    def top_k(self, terms: Sequence[Term], key_cols: Sequence[int], k: int, descending: bool = False, proj: Sequence[int] = (),
+              want: int = N.WANT_POSITIONS | N.WANT_COLUMNS | N.WANT_HOST) -> "Result":
+        """ORDER BY key_cols LIMIT k over the rows that satisfy the CNF: the first min(k, Q) rows of sort()'s order over
+        the Q qualifying rows (ties by ascending position in both directions), with their positions and projected fields."""
+        tarr, nt, keep = pack_terms(terms)
+        karr = (C.c_int32 * max(len(key_cols), 1))(*key_cols)
+        parr = (C.c_int32 * max(len(proj), 1))(*proj)
+        h = C.c_void_p()
+        N.check(N.lib().mbc_topk(self._h, tarr, nt, karr, len(key_cols), 1 if descending else 0, k, parr, len(proj), want,
+                                 C.byref(h)))
+        del keep
+        return Result(self.ctx, h, [self.coldescs[c] for c in proj], want, 0)
+
     # ---- bitmap indexes --------------------------------------------------------------------
     def bitmap_build(self, col: int) -> None:
         N.check(N.lib().mbc_bitmap_build(self._h, col))

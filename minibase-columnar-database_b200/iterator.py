@@ -322,6 +322,24 @@ class ColumnarFileScan(Iterator):
         finally:
             res.close()
 
+    def top_k(self, key_fields: Sequence[int], k: int, descending: bool = False) -> list:
+        """ORDER BY the 0-based columns key_fields LIMIT k over the rows OutputFilter selects: one (position, (projected
+        field values...)) pair per row in key order, ties by ascending position; the fields are those of perm_mat, ints
+        as int, reals as float, strings as str."""
+        cols = [fs.offset - 1 for fs in self.perm_mat]
+        res = self.f.table.top_k(flatten_condexpr(self.OutputFilter), list(key_fields), k, descending, proj=cols)
+        try:
+            fields = []
+            for i, col in enumerate(cols):
+                vals = res.column(i)
+                if self.f.attrTypes[col].attrType == AttrType.attrString:
+                    fields.append([bytes(r).split(b"\0", 1)[0].decode("utf-8") for r in vals])
+                else:
+                    fields.append(vals.tolist())
+            return [(int(p), tuple(f[g] for f in fields)) for g, p in enumerate(res.positions().tolist())]
+        finally:
+            res.close()
+
 
 class _ColumnsScan(Iterator):
     """Shared body of ColumnarColumnScan / ColumnarColumnsScan (SURVEY.md 8f rank 1): the predicate is evaluated over a
