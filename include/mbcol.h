@@ -287,9 +287,18 @@ int32_t mbc_group_aggregate(mbc_table* t, const mbc_term* terms, int32_t nterms,
  *                mbc_shard_gather(sh, result, beside_next_scan)   asynchronous; then mbc_shard_fence(sh) before the
  *                                                                 result is freed when beside_next_scan != 0
  *   root:        mbc_shard_collect(sh, &total, counts)       waits for every rank's rows; mbc_shard_agg folds aggregates;
- *                mbc_shard_read / mbc_shard_window_device     the gathered rows;   mbc_shard_release(sh) ends the step.
+ *                mbc_shard_read / mbc_shard_window_device     the gathered rows;
+ *                mbc_shard_topk / mbc_shard_group             ORDER BY ... LIMIT k / GROUP BY over the gathered rows;
+ *                mbc_shard_release(sh) ends the step.
  * Every rank must call mbc_shard_gather exactly once per step (the calls are matched by a step counter), with results
- * of the same projection; the root must release a step before the ranks can gather the step after the next one. */
+ * of the same projection; the root must release a step before the ranks can gather the step after the next one.
+ * What a result puts in the window (its shape must match the window's columns and strides, else MBC_ERR_ARG):
+ *   mbc_scan / mbc_scan_host / mbc_bitmap_scan: positions, projected columns, count and aggregates (mbc_shard_agg).
+ *   mbc_topk / mbc_sort (MBC_WANT_POSITIONS): positions and projected columns in the rank's sort order, and the count.
+ *   mbc_group_aggregate (MBC_WANT_POSITIONS | MBC_WANT_COLUMNS, plus MBC_WANT_AGG with aggregates): per group its lowest
+ *       position, then the window columns are the key columns followed by one column of stride 8 per aggregate (the raw
+ *       int64 / double values).  More than 16 key columns + aggregates: MBC_ERR_UNSUPPORTED.
+ *   mbc_bitmap_join (position pairs): MBC_ERR_ARG. */
 typedef struct mbc_shard mbc_shard;
 #define MBC_IPC_HANDLE_BYTES 64
 int32_t mbc_shard_create(mbc_ctx* ctx, int32_t rank, int32_t world, mbc_shard** out);
@@ -319,6 +328,30 @@ int32_t mbc_shard_window_device(const mbc_shard* sh, void** d_positions, int32_t
 /* copy rows [first_row, first_row + nrows) of the gathered positions (col = -1, int64) or of column `col` to the host */
 int32_t mbc_shard_read(mbc_shard* root, int32_t col, int64_t first_row, int64_t nrows, void* host_out);
 int32_t mbc_shard_release(mbc_shard* root);
+/* ORDER BY ... LIMIT k over the rows the ranks gathered from mbc_topk (the same keys, direction and a k' >= k on every rank)
+ * or from mbc_sort (k >= the total is then a sharded ORDER BY).  descs: type / width of every window column;
+ * key_fields / proj_fields: window column indices.  The result is the first min(k, total) rows of mbc_topk's order over the
+ * whole sharded table (equal keys in ascending global position, in both directions; -0.0 and +0.0 one key): positions
+ * (global), projected fields, Tuple bytes and host copies as mbc_topk.
+ *   Root only, after mbc_shard_collect and before mbc_shard_release: else MBC_ERR_ARG.  Returns after its kernels have
+ *   finished reading the window.
+ *   k < 0, a field index out of range or a desc whose stride differs from the window's: MBC_ERR_ARG.  k == 0: empty.
+ *   MBC_WANT_AGG / MBC_WANT_BITMAP, > 2^32 - 1 gathered rows: MBC_ERR_UNSUPPORTED. */
+int32_t mbc_shard_topk(mbc_shard* root, const mbc_coldesc* descs, const int32_t* key_fields, int32_t nkeys,
+                       int32_t descending, int64_t k, const int32_t* proj_fields, int32_t nproj, uint32_t want,
+                       mbc_result** out);
+/* GROUP BY over the grouped results the ranks gathered (mbc_group_aggregate with the same keys and aggregates on every
+ * rank).  key_descs: the nkeys key columns; agg_kinds / agg_types: the kind (MBC_AGG_*) and the aggregated column's type
+ * of each aggregate, as the ranks asked for them.  The result has mbc_group_aggregate's contract over the whole sharded
+ * table (mbc_result_count / _column / _positions / _group_agg): a global group's COUNT and SUM are sums of the ranks'
+ * partials, MIN / MAX their min / max, folded in rank order (so the result is the same from run to run); its position and
+ * key values are those of the lowest rank holding the group.
+ *   Root only, after mbc_shard_collect and before mbc_shard_release: else MBC_ERR_ARG.  Returns after its kernels have
+ *   finished reading the window.
+ *   A window that is not nkeys key columns of these descs + nagg columns of stride 8: MBC_ERR_ARG.
+ *   MBC_WANT_TUPLES / MBC_WANT_BITMAP, nkeys + nagg > 16, > 2^32 - 1 gathered rows: MBC_ERR_UNSUPPORTED. */
+int32_t mbc_shard_group(mbc_shard* root, const mbc_coldesc* key_descs, int32_t nkeys, const int32_t* agg_kinds,
+                        const int32_t* agg_types, int32_t nagg, uint32_t want, mbc_result** out);
 
 /* ---- results -------------------------------------------------------------------------- */
 /* A device-resident result of mbc_scan (no MBC_WANT_HOST / MBC_WANT_TUPLES) completes asynchronously:

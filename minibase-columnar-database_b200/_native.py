@@ -125,6 +125,10 @@ _SIGNATURES = {
     "mbc_shard_window_device": (C.c_int32, [_VP, C.POINTER(_VP), C.c_int32, C.POINTER(_VP)]),
     "mbc_shard_read": (C.c_int32, [_VP, C.c_int32, C.c_int64, C.c_int64, _VP]),
     "mbc_shard_release": (C.c_int32, [_VP]),
+    "mbc_shard_topk": (C.c_int32, [_VP, C.POINTER(mbc_coldesc), C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.c_int64,
+                                   C.POINTER(C.c_int32), C.c_int32, C.c_uint32, C.POINTER(_VP)]),
+    "mbc_shard_group": (C.c_int32, [_VP, C.POINTER(mbc_coldesc), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                                    C.c_int32, C.c_uint32, C.POINTER(_VP)]),
 }
 IPC_HANDLE_BYTES = 64
 

@@ -436,7 +436,7 @@ const uint8_t* mbc_result_tuples(const mbc_result* r, int32_t* tuple_len) {
 }
 
 int32_t mbc_result_agg(const mbc_result* r, int32_t i, int64_t* as_i64, double* as_f64, int32_t* valid) {
-    if (r && r->grouped) MBC_FAIL(MBC_ERR_ARG, "mbc_result_agg: a grouped result has one value per group (mbc_result_group_agg)");
+    if (r && r->kind == mbc_result::kGrouped) MBC_FAIL(MBC_ERR_ARG, "mbc_result_agg: a grouped result has one value per group (mbc_result_group_agg)");
     if (!r || i < 0 || i >= (int)r->aggs.size()) MBC_FAIL(MBC_ERR_ARG, "mbc_result_agg: index %d of %d", i,
                                                           r ? (int)r->aggs.size() : 0);
     MBC_TRY(result_finalize(const_cast<mbc_result*>(r)));
@@ -447,7 +447,7 @@ int32_t mbc_result_agg(const mbc_result* r, int32_t i, int64_t* as_i64, double* 
 }
 
 int32_t mbc_result_group_agg(const mbc_result* r, int32_t i, const int64_t** as_i64, const double** as_f64) {
-    if (!r || !r->grouped) MBC_FAIL(MBC_ERR_ARG, "mbc_result_group_agg: not a result of mbc_group_aggregate");
+    if (!r || r->kind != mbc_result::kGrouped) MBC_FAIL(MBC_ERR_ARG, "mbc_result_group_agg: not a grouped result");
     if (i < 0 || i >= (int)r->group_aggs.size())
         MBC_FAIL(MBC_ERR_ARG, "mbc_result_group_agg: index %d of %d aggregates on the host (MBC_WANT_AGG | MBC_WANT_HOST)", i,
                  (int)r->group_aggs.size());

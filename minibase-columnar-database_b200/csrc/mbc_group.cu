@@ -36,6 +36,7 @@ struct GroupAggs {
     int32_t kind[kMaxAgg];
     int32_t type[kMaxAgg];     // column type; MBC_ATTR_INTEGER for COUNT
     int32_t n;
+    int32_t partials;          // every src holds 8-byte raw aggregates (int64, or double for a real SUM / MIN / MAX)
 };
 
 // head[i] = 1 where sorted row rows[i] starts a group: some key differs from that of rows[i-1].  Reals compare as floats,
@@ -62,7 +63,7 @@ __global__ void __launch_bounds__(256) group_heads_kernel(const uint32_t* __rest
 
 // ---- segmented fold ---------------------------------------------------------------------------------------------
 enum { kOpAdd = 0, kOpMin = 1, kOpMax = 2 };
-enum { kSrcOne = 0, kSrcInt = 1, kSrcReal = 2 };
+enum { kSrcOne = 0, kSrcInt = 1, kSrcReal = 2, kSrcPartial = 3 };
 
 template <typename T, int OP> __device__ __forceinline__ T fold_identity() {
     using L = std::numeric_limits<T>;
@@ -78,6 +79,7 @@ template <typename T, int OP> __device__ __forceinline__ T fold_op(T a, T b) {
 template <typename T, int SRC> __device__ __forceinline__ T fold_load(const void* src, uint32_t row) {
     if (SRC == kSrcOne) return (T)1;
     if (SRC == kSrcInt) return (T)__ldg(reinterpret_cast<const int32_t*>(src) + row);
+    if (SRC == kSrcPartial) return __ldg(reinterpret_cast<const T*>(src) + row);   // a COUNT partial is an int64 to add
     return (T)__ldg(reinterpret_cast<const float*>(src) + row);
 }
 template <typename T> __device__ __forceinline__ unsigned long long fold_raw(T v) {
@@ -167,9 +169,10 @@ __device__ void fold_chunk(const FoldThread& ft, const void* src, unsigned long 
 }
 
 template <typename T, int OP, int SRC>
-__device__ __forceinline__ void fold_chunk_smem(const FoldThread& ft, const void* src, unsigned long long* out,
+__device__ __forceinline__ void fold_chunk_smem(const FoldThread& ft, const void* src, bool partial, unsigned long long* out,
                                                 unsigned long long* parts, int* s_flag, unsigned long long* s_raw) {
-    fold_chunk<T, OP, SRC>(ft, src, out, parts, s_flag, reinterpret_cast<T*>(s_raw));
+    if (partial) fold_chunk<T, OP, kSrcPartial>(ft, src, out, parts, s_flag, reinterpret_cast<T*>(s_raw));
+    else fold_chunk<T, OP, SRC>(ft, src, out, parts, s_flag, reinterpret_cast<T*>(s_raw));
 }
 
 // aggregate a of the groups: out[a * G + g] raw (int64, or the bits of a double for a real SUM / MIN / MAX)
@@ -207,20 +210,20 @@ __global__ void __launch_bounds__(kGroupThreads) group_fold_kernel(const uint32_
         unsigned long long* o = out + (size_t)a * G;
         unsigned long long* p = cparts + (size_t)a * 2 * nchunks;
         const void* src = aggs.src[a];
-        const bool real = aggs.type[a] == MBC_ATTR_REAL;
+        const bool real = aggs.type[a] == MBC_ATTR_REAL, pt = aggs.partials != 0;
         switch (aggs.kind[a]) {
-            case MBC_AGG_COUNT: fold_chunk_smem<long long, kOpAdd, kSrcOne>(ft, src, o, p, s_flag, s_raw); break;
+            case MBC_AGG_COUNT: fold_chunk_smem<long long, kOpAdd, kSrcOne>(ft, src, pt, o, p, s_flag, s_raw); break;
             case MBC_AGG_SUM:
-                if (real) fold_chunk_smem<double, kOpAdd, kSrcReal>(ft, src, o, p, s_flag, s_raw);
-                else fold_chunk_smem<long long, kOpAdd, kSrcInt>(ft, src, o, p, s_flag, s_raw);
+                if (real) fold_chunk_smem<double, kOpAdd, kSrcReal>(ft, src, pt, o, p, s_flag, s_raw);
+                else fold_chunk_smem<long long, kOpAdd, kSrcInt>(ft, src, pt, o, p, s_flag, s_raw);
                 break;
             case MBC_AGG_MIN:
-                if (real) fold_chunk_smem<double, kOpMin, kSrcReal>(ft, src, o, p, s_flag, s_raw);
-                else fold_chunk_smem<long long, kOpMin, kSrcInt>(ft, src, o, p, s_flag, s_raw);
+                if (real) fold_chunk_smem<double, kOpMin, kSrcReal>(ft, src, pt, o, p, s_flag, s_raw);
+                else fold_chunk_smem<long long, kOpMin, kSrcInt>(ft, src, pt, o, p, s_flag, s_raw);
                 break;
             default:
-                if (real) fold_chunk_smem<double, kOpMax, kSrcReal>(ft, src, o, p, s_flag, s_raw);
-                else fold_chunk_smem<long long, kOpMax, kSrcInt>(ft, src, o, p, s_flag, s_raw);
+                if (real) fold_chunk_smem<double, kOpMax, kSrcReal>(ft, src, pt, o, p, s_flag, s_raw);
+                else fold_chunk_smem<long long, kOpMax, kSrcInt>(ft, src, pt, o, p, s_flag, s_raw);
                 break;
         }
     }
@@ -291,86 +294,43 @@ static int grid_for(const mbc_ctx* ctx, int64_t n) {
     return (int)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, (int64_t)ctx->sm_count * 8));
 }
 
-}  // namespace mbc
-
-using namespace mbc;
-
-extern "C" int32_t mbc_group_aggregate(mbc_table* t, const mbc_term* terms, int32_t nterms, const int32_t* key_cols, int32_t nkeys,
-                                       const mbc_aggspec* aggs, int32_t nagg, uint32_t want, mbc_result** out) {
-    if (!t || !out || !key_cols || nkeys <= 0 || (nagg > 0 && !aggs) || nagg < 0)
-        MBC_FAIL(MBC_ERR_ARG, "mbc_group_aggregate: bad argument");
-    *out = nullptr;
-    if (want & (MBC_WANT_TUPLES | MBC_WANT_BITMAP))
-        MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_group_aggregate: MBC_WANT_TUPLES / MBC_WANT_BITMAP are not available for groups");
-    if (nkeys > kMaxTerms) MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_group_aggregate: %d key columns (max %d)", nkeys, kMaxTerms);
-    if (nagg > kMaxAgg) MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_group_aggregate: %d aggregates (max %d)", nagg, kMaxAgg);
+int32_t group_rows(mbc_ctx* ctx, uint32_t* rows, int64_t n, const Column* keys, int32_t nkeys, const GroupAggSpec* aggs, int32_t nagg,
+                   bool partials, const int64_t* pos, int64_t pos_base, mbc_result* r) {
+    const uint32_t want = r->want;
     GroupKeys gk{};
     gk.n = nkeys;
     for (int k = 0; k < nkeys; ++k) {
-        if (key_cols[k] < 0 || key_cols[k] >= (int)t->cols.size())
-            MBC_FAIL(MBC_ERR_ARG, "mbc_group_aggregate: key column %d out of range", key_cols[k]);
-        const Column& c = t->cols[key_cols[k]];
-        gk.d[k] = c.d;
-        gk.stride[k] = c.stride;
-        gk.type[k] = c.type;
+        gk.d[k] = keys[k].d;
+        gk.stride[k] = keys[k].stride;
+        gk.type[k] = keys[k].type;
     }
     GroupAggs ga{};
     ga.n = (want & MBC_WANT_AGG) ? nagg : 0;
-    for (int a = 0; a < nagg; ++a) {
-        const int kind = aggs[a].kind, col = aggs[a].col;
-        if (kind < MBC_AGG_COUNT || kind > MBC_AGG_MAX) MBC_FAIL(MBC_ERR_ARG, "mbc_group_aggregate: aggregate %d: unknown kind %d", a, kind);
-        ga.kind[a] = kind;
-        ga.type[a] = MBC_ATTR_INTEGER;
-        if (kind == MBC_AGG_COUNT) continue;
-        if (col < 0 || col >= (int)t->cols.size()) MBC_FAIL(MBC_ERR_ARG, "mbc_group_aggregate: aggregate %d: column %d out of range", a, col);
-        if (t->cols[col].type == MBC_ATTR_STRING) MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_group_aggregate: aggregate %d over a string column", a);
-        ga.src[a] = t->cols[col].d;
-        ga.type[a] = t->cols[col].type;
+    ga.partials = partials ? 1 : 0;
+    for (int a = 0; a < ga.n; ++a) {
+        ga.src[a] = aggs[a].src;
+        ga.kind[a] = aggs[a].kind;
+        ga.type[a] = aggs[a].type;
     }
-    if (t->nrows > (int64_t)UINT32_MAX) MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_group_aggregate: more than 2^32 rows in one table");
-    mbc_ctx* ctx = t->ctx;
-    MBC_CUDA(cudaSetDevice(ctx->device));
-
-    // the qualifying rows in position order (the predicate checks its terms)
-    mbc_result* sel = nullptr;
-    ScanRequest rq;
-    rq.table = t;
-    rq.terms = terms;
-    rq.nterms = nterms;
-    rq.want = MBC_WANT_POSITIONS;
-    MBC_TRY(run_scan(rq, &sel));
-    const int64_t n = sel->count;
-    split_timing(ctx);                                      // the scan's kernels count, the host wait in between does not
-    begin_timing(ctx);
-
-    mbc_result* r = new mbc_result();
-    r->ctx = ctx;
-    ctx_retain(ctx);
-    r->want = want;
-    r->nrows = t->nrows;
-    r->grouped = true;
-    uint32_t *rows = nullptr, *head = nullptr, *bits = nullptr, *start = nullptr, *head_row = nullptr;
+    r->kind = mbc_result::kGrouped;
+    r->group_nagg = ga.n;
+    uint32_t *head = nullptr, *bits = nullptr, *start = nullptr, *head_row = nullptr;
     unsigned long long *group_of = nullptr, *parts = nullptr;
     auto release = [&]() {
-        for (void* p : {(void*)rows, (void*)head, (void*)bits, (void*)start, (void*)head_row, (void*)group_of, (void*)parts}) dev_free(ctx, p);
-        mbc_result_free(sel);
+        for (void* p : {(void*)head, (void*)bits, (void*)start, (void*)head_row, (void*)group_of, (void*)parts}) dev_free(ctx, p);
     };
     auto fail = [&](int32_t s) {
         release();
-        mbc_result_free(r);
         return s;
     };
 #define GTRY(x) do { int32_t _s = (x); if (_s != MBC_OK) return fail(_s); } while (0)
-#define GCUDA(x) do { cudaError_t _e = (x); if (_e != cudaSuccess) return fail((set_error("mbc_group_aggregate: %s", cudaGetErrorString(_e)), MBC_ERR_CUDA)); } while (0)
+#define GCUDA(x) do { cudaError_t _e = (x); if (_e != cudaSuccess) return fail((set_error("group: %s", cudaGetErrorString(_e)), MBC_ERR_CUDA)); } while (0)
     const int grid = grid_for(ctx, n);
     GTRY(dev_alloc(ctx, (void**)&group_of, (size_t)(n + 1) * 8, false));
     if (n > 0) {
-        GTRY(dev_alloc(ctx, (void**)&rows, (size_t)n * 4, false));
         GTRY(dev_alloc(ctx, (void**)&head, (size_t)n * 4, false));            // sort keys, then the head flags
         GTRY(dev_alloc(ctx, (void**)&bits, 8, false));
-        sort_rows_from_positions_kernel<<<grid, 256, 0, ctx->stream>>>(sel->d_pos, n, t->pos_base, rows);
-        ctx->launches++;
-        for (int k = nkeys - 1; k >= 0; --k) GTRY(sort_rows_by_column(ctx, rows, n, t->cols[key_cols[k]], false, head, bits));
+        for (int k = nkeys - 1; k >= 0; --k) GTRY(sort_rows_by_column(ctx, rows, n, keys[k], false, head, bits));
         group_heads_kernel<<<grid, 256, 0, ctx->stream>>>(rows, n, gk, head);
         ctx->launches++;
     }
@@ -386,15 +346,16 @@ extern "C" int32_t mbc_group_aggregate(mbc_table* t, const mbc_term* terms, int3
         sparse_run_starts_kernel<<<grid, 256, 0, ctx->stream>>>(head, group_of, rows, n, start, head_row);
         ctx->launches++;
     }
-    // a group's head row is its lowest qualifying position: the sort is stable over rows in position order
+    // a group's head row is its first row id: the sort is stable over row ids in position order
     if ((want & MBC_WANT_POSITIONS) && G > 0) {
         GTRY(dev_alloc(ctx, (void**)&r->d_pos, (size_t)G * 8, false));
-        sort_positions_kernel<<<grid_for(ctx, (int64_t)G), 256, 0, ctx->stream>>>(head_row, (int64_t)G, t->pos_base, r->d_pos);
+        if (pos) sort_gather_kernel<<<grid_for(ctx, (int64_t)G), 256, 0, ctx->stream>>>(head_row, (int64_t)G, pos, 8, r->d_pos);
+        else sort_positions_kernel<<<grid_for(ctx, (int64_t)G), 256, 0, ctx->stream>>>(head_row, (int64_t)G, pos_base, r->d_pos);
         ctx->launches++;
     }
     if (want & MBC_WANT_COLUMNS) {
         for (int k = 0; k < nkeys; ++k) {
-            const Column& col = t->cols[key_cols[k]];
+            const Column& col = keys[k];
             mbc_result::Col rc{col.type, col.width, col.stride, nullptr, nullptr};
             GTRY(dev_alloc(ctx, &rc.d, (size_t)std::max<unsigned long long>(G, 1) * col.stride, false));
             r->cols.push_back(rc);
@@ -441,6 +402,74 @@ extern "C" int32_t mbc_group_aggregate(mbc_table* t, const mbc_term* terms, int3
 #undef GTRY
 #undef GCUDA
     release();
+    return MBC_OK;
+}
+
+}  // namespace mbc
+
+using namespace mbc;
+
+extern "C" int32_t mbc_group_aggregate(mbc_table* t, const mbc_term* terms, int32_t nterms, const int32_t* key_cols, int32_t nkeys,
+                                       const mbc_aggspec* aggs, int32_t nagg, uint32_t want, mbc_result** out) {
+    if (!t || !out || !key_cols || nkeys <= 0 || (nagg > 0 && !aggs) || nagg < 0)
+        MBC_FAIL(MBC_ERR_ARG, "mbc_group_aggregate: bad argument");
+    *out = nullptr;
+    if (want & (MBC_WANT_TUPLES | MBC_WANT_BITMAP))
+        MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_group_aggregate: MBC_WANT_TUPLES / MBC_WANT_BITMAP are not available for groups");
+    if (nkeys > kMaxTerms) MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_group_aggregate: %d key columns (max %d)", nkeys, kMaxTerms);
+    if (nagg > kMaxAgg) MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_group_aggregate: %d aggregates (max %d)", nagg, kMaxAgg);
+    Column keys[kMaxTerms];
+    for (int k = 0; k < nkeys; ++k) {
+        if (key_cols[k] < 0 || key_cols[k] >= (int)t->cols.size())
+            MBC_FAIL(MBC_ERR_ARG, "mbc_group_aggregate: key column %d out of range", key_cols[k]);
+        keys[k] = t->cols[key_cols[k]];
+    }
+    GroupAggSpec specs[kMaxAgg] = {};
+    for (int a = 0; a < nagg; ++a) {
+        const int kind = aggs[a].kind, col = aggs[a].col;
+        if (kind < MBC_AGG_COUNT || kind > MBC_AGG_MAX) MBC_FAIL(MBC_ERR_ARG, "mbc_group_aggregate: aggregate %d: unknown kind %d", a, kind);
+        specs[a].kind = kind;
+        specs[a].type = MBC_ATTR_INTEGER;
+        if (kind == MBC_AGG_COUNT) continue;
+        if (col < 0 || col >= (int)t->cols.size()) MBC_FAIL(MBC_ERR_ARG, "mbc_group_aggregate: aggregate %d: column %d out of range", a, col);
+        if (t->cols[col].type == MBC_ATTR_STRING) MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_group_aggregate: aggregate %d over a string column", a);
+        specs[a].src = t->cols[col].d;
+        specs[a].type = t->cols[col].type;
+    }
+    if (t->nrows > (int64_t)UINT32_MAX) MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_group_aggregate: more than 2^32 rows in one table");
+    mbc_ctx* ctx = t->ctx;
+    MBC_CUDA(cudaSetDevice(ctx->device));
+
+    // the qualifying rows in position order (the predicate checks its terms)
+    mbc_result* sel = nullptr;
+    ScanRequest rq;
+    rq.table = t;
+    rq.terms = terms;
+    rq.nterms = nterms;
+    rq.want = MBC_WANT_POSITIONS;
+    MBC_TRY(run_scan(rq, &sel));
+    const int64_t n = sel->count;
+    split_timing(ctx);                                      // the scan's kernels count, the host wait in between does not
+    begin_timing(ctx);
+
+    mbc_result* r = new mbc_result();
+    r->ctx = ctx;
+    ctx_retain(ctx);
+    r->want = want;
+    r->nrows = t->nrows;
+    uint32_t* rows = nullptr;
+    int32_t s = dev_alloc(ctx, (void**)&rows, (size_t)std::max<int64_t>(n, 1) * 4, false);
+    if (s == MBC_OK && n > 0) {
+        sort_rows_from_positions_kernel<<<grid_for(ctx, n), 256, 0, ctx->stream>>>(sel->d_pos, n, t->pos_base, rows);
+        ctx->launches++;
+    }
+    if (s == MBC_OK) s = group_rows(ctx, rows, n, keys, nkeys, specs, nagg, false, nullptr, t->pos_base, r);
+    dev_free(ctx, rows);
+    mbc_result_free(sel);
+    if (s != MBC_OK) {
+        mbc_result_free(r);
+        return s;
+    }
     *out = r;
     return MBC_OK;
 }

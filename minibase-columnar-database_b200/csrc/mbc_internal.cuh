@@ -153,6 +153,15 @@ struct mbc_table {
 };
 
 struct mbc_result {
+    // what the buffers hold, set by the call that made the result (mbc_shard_gather carries each kind differently)
+    enum Kind : int32_t {
+        kUnset = 0,
+        kScan,      // mbc_scan / mbc_scan_host / mbc_bitmap_scan: d_aggs = kMaxAgg raw aggregates + the count
+        kRows,      // mbc_sort / mbc_topk / mbc_shard_topk: positions + fields in sort order, no d_aggs
+        kGrouped,   // mbc_group_aggregate / mbc_shard_group: one row per group, d_aggs = nagg x count raw values
+        kJoin,      // mbc_bitmap_join: position pairs
+    };
+    Kind kind = kUnset;
     mbc_ctx* ctx = nullptr;
     uint32_t want = 0;
     int64_t count = 0;
@@ -177,8 +186,8 @@ struct mbc_result {
     // aggregates
     struct Agg { int32_t kind, type; int64_t i; double f; int32_t valid; };
     std::vector<Agg> aggs;
-    // mbc_group_aggregate: one row per group; d_aggs holds nagg x count raw values, group_aggs their host decode
-    bool grouped = false;
+    // kGrouped: d_aggs holds group_nagg x count raw values, group_aggs their host decode
+    int32_t group_nagg = 0;
     struct GroupAgg { std::vector<int64_t> i; std::vector<double> f; };
     std::vector<GroupAgg> group_aggs;
     // Deferred completion (device-resident results of mbc_scan): the call returns with its kernels and the small
@@ -245,7 +254,9 @@ __global__ void __launch_bounds__(256) sort_key_bits_kernel(const uint32_t* __re
 // rows[i] = pos[i] - base
 __global__ void __launch_bounds__(256) sort_rows_from_positions_kernel(const int64_t* __restrict__ pos, int64_t n, int64_t base,
                                                                       uint32_t* __restrict__ rows);
-// out row i = column row rows[i] (stride bytes, a multiple of 4)
+// rows[i] = i
+__global__ void __launch_bounds__(256) sort_iota_kernel(int64_t n, uint32_t* __restrict__ rows);
+// out row i = column row rows[i] (stride bytes, a multiple of 4; stride 8 gathers int64 positions)
 __global__ void __launch_bounds__(256) sort_gather_kernel(const uint32_t* __restrict__ rows, int64_t n, const void* src, int stride, void* dst);
 // pos[i] = base + rows[i]
 __global__ void __launch_bounds__(256) sort_positions_kernel(const uint32_t* __restrict__ rows, int64_t n, int64_t base, int64_t* __restrict__ pos);
@@ -256,5 +267,19 @@ __global__ void __launch_bounds__(256) sparse_run_starts_kernel(const uint32_t* 
 // stable reorder of the row ids `rows` by column c (every 32-bit word of its key, least significant first), so rows
 // with equal keys keep their order; keys (n words) and bits (2 words) are scratch
 int32_t sort_rows_by_column(mbc_ctx* ctx, uint32_t* rows, int64_t n, const Column& c, bool descending, uint32_t* keys, uint32_t* bits);
+
+// ---- GROUP BY over row ids, shared by mbc_group_aggregate and mbc_shard_group (mbc_group.cu) ------------------------
+struct GroupAggSpec {
+    int32_t kind;              // MBC_AGG_*
+    int32_t type;              // type of the aggregated column (MBC_ATTR_INTEGER for COUNT)
+    const void* src;           // per row id: int32 / float32 column values, or 8-byte raw partials when `partials`
+};
+// Groups the n row ids `rows` (sorted in place) by the key columns, ascending, equal keys in row-id order.  Row id i's
+// position is pos[i] when pos is not NULL, else pos_base + i; each group's positions / key values are those of its first
+// row id.  `partials`: every source holds raw aggregates of earlier groupings (a COUNT partial is added).  Fills r (ctx,
+// want set by the caller): count, d_pos, cols, d_aggs, group_nagg, group_aggs; host copies per r->want.  Ends the caller's
+// timed segment (begin_timing) after the kernels, and returns after they have finished.
+int32_t group_rows(mbc_ctx* ctx, uint32_t* rows, int64_t n, const Column* keys, int32_t nkeys, const GroupAggSpec* aggs, int32_t nagg,
+                   bool partials, const int64_t* pos, int64_t pos_base, mbc_result* r);
 
 }  // namespace mbc

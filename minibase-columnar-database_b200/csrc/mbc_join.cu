@@ -943,6 +943,7 @@ extern "C" int32_t mbc_bitmap_join(mbc_table* outer, mbc_table* inner, const mbc
     const bool want_pairs = (want & (MBC_WANT_POSITIONS | MBC_WANT_COLUMNS | MBC_WANT_TUPLES)) != 0;
 
     mbc_result* r = new mbc_result();
+    r->kind = mbc_result::kJoin;
     r->ctx = ctx;
     ctx_retain(ctx);
     r->want = want;

@@ -462,6 +462,7 @@ static int32_t prepare_job(const mbc_table* schema, const ScanRequest& rq, int64
 
     mbc_result* r = new mbc_result();
     job->r = r;
+    r->kind = mbc_result::kScan;
     r->ctx = ctx;
     ctx_retain(ctx);
     r->want = rq.want;

@@ -241,6 +241,8 @@ struct mbc_shard {
     long long* d_off = nullptr;
     cudaEvent_t ev_off = nullptr;
     int64_t total = 0, dropped = 0;
+    unsigned long long collected = 0;   // the step mbc_shard_collect completed, until mbc_shard_release (0: none)
+    unsigned long long* d_count_block = nullptr;   // zero aggregates + the count of a row or grouped result (shard_publish_kernel)
     std::vector<int64_t> counts;
     int push_ctas = 0;
 };
@@ -273,6 +275,35 @@ static int32_t set_shape(mbc_shard* s, int64_t capacity_rows, int32_t ncols, con
     return MBC_OK;
 }
 
+// ---- root-side merges of the gathered rows ----------------------------------------------------------------------------
+// The window's rows are the input, row id i = window row i; rank order is position order, so a stable sort of the row ids
+// keeps equal keys in ascending global position.
+
+static int32_t merge_check(const mbc_shard* s, const char* fn) {
+    if (!s || !s->owned) MBC_FAIL(MBC_ERR_ARG, "%s: only the window's owner merges", fn);
+    if (s->epoch == 0 || s->collected != s->epoch) MBC_FAIL(MBC_ERR_ARG, "%s: no collected step (mbc_shard_collect first, mbc_shard_release after)", fn);
+    if (s->total > (int64_t)UINT32_MAX) MBC_FAIL(MBC_ERR_UNSUPPORTED, "%s: %lld gathered rows (max 2^32 - 1)", fn, (long long)s->total);
+    return MBC_OK;
+}
+
+// window column c of the collected step as a table column of type/width d
+static int32_t window_column(const mbc_shard* s, const char* fn, int c, const mbc_coldesc& d, Column* out) {
+    int stride = 0;
+    if ((d.type == MBC_ATTR_INTEGER || d.type == MBC_ATTR_REAL) && d.width == 4) stride = 4;
+    else if (d.type == MBC_ATTR_STRING && d.width > 0 && d.width <= kMaxStrStride) stride = str_stride(d.width);
+    if (stride == 0) MBC_FAIL(MBC_ERR_ARG, "%s: column %d: type %d width %d", fn, c, d.type, d.width);
+    if (stride != s->strides[c]) MBC_FAIL(MBC_ERR_ARG, "%s: column %d has stride %d, the window %d", fn, c, stride, s->strides[c]);
+    out->type = d.type;
+    out->width = d.width;
+    out->stride = stride;
+    out->d = s->win + s->off_col[s->epoch % kShardSlots][c];
+    return MBC_OK;
+}
+
+static int merge_grid(const mbc_ctx* ctx, int64_t n) {
+    return (int)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, (int64_t)ctx->sm_count * 8));
+}
+
 extern "C" {
 
 int32_t mbc_shard_create(mbc_ctx* ctx, int32_t rank, int32_t world, mbc_shard** out) {
@@ -295,7 +326,9 @@ int32_t mbc_shard_create(mbc_ctx* ctx, int32_t rank, int32_t world, mbc_shard** 
         cudaEventCreateWithFlags(&s->ev_off, cudaEventDisableTiming) != cudaSuccess ||
         cudaHostAlloc((void**)&s->h_off, 64, cudaHostAllocMapped) != cudaSuccess ||
         cudaHostGetDevicePointer((void**)&s->d_off, s->h_off, 0) != cudaSuccess ||
-        cudaMalloc((void**)&s->d_blocks_done, 64) != cudaSuccess || cudaMemset(s->d_blocks_done, 0, 64) != cudaSuccess) {
+        cudaMalloc((void**)&s->d_blocks_done, 64) != cudaSuccess || cudaMemset(s->d_blocks_done, 0, 64) != cudaSuccess ||
+        cudaMalloc((void**)&s->d_count_block, (kMaxAgg + 1) * 8) != cudaSuccess ||
+        cudaMemset(s->d_count_block, 0, (kMaxAgg + 1) * 8) != cudaSuccess) {
         set_error("mbc_shard_create: %s", cudaGetErrorString(cudaGetLastError()));
         mbc_shard_free(s);
         return MBC_ERR_CUDA;
@@ -314,6 +347,7 @@ void mbc_shard_free(mbc_shard* s) {
         else if (s->ipc) cudaIpcCloseMemHandle(s->win);
     }
     if (s->d_blocks_done) cudaFree(s->d_blocks_done);
+    if (s->d_count_block) cudaFree(s->d_count_block);
     if (s->d_summary) cudaFree(s->d_summary);
     if (s->h_summary) cudaFreeHost(s->h_summary);
     if (s->h_off) cudaFreeHost(s->h_off);
@@ -377,9 +411,42 @@ int32_t mbc_shard_window_attach(mbc_shard* s, const mbc_shard* root) {
 int32_t mbc_shard_gather(mbc_shard* s, const mbc_result* r, int32_t beside_next_scan) {
     if (!s || !s->win || !r) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_gather: no window / result");
     if (r->ctx != s->ctx) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_gather: the result belongs to another context");
-    if ((int)r->cols.size() != s->ncols) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_gather: result has %zu columns, window %d", r->cols.size(), s->ncols);
+    // the window columns this result fills, and where its count (after kMaxAgg aggregates) is read from
+    const void* src[kMaxProj];
+    int32_t src_stride[kMaxProj];
+    int nsrc = (int)r->cols.size();
+    for (int c = 0; c < nsrc && c < kMaxProj; ++c) {
+        src[c] = r->cols[c].d;
+        src_stride[c] = r->cols[c].stride;
+    }
+    bool own_count = false;             // rows / groups: the count comes from the host, through d_count_block
+    switch (r->kind) {
+        case mbc_result::kScan:
+            break;
+        case mbc_result::kRows:
+            if (!(r->want & MBC_WANT_POSITIONS)) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_gather: a sorted result needs MBC_WANT_POSITIONS");
+            own_count = true;
+            break;
+        case mbc_result::kGrouped: {
+            // key columns, then one 8-byte column per aggregate: aggregate a's values are the block d_aggs + a * count
+            if (nsrc + r->group_nagg > kMaxProj)
+                MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_shard_gather: %d key columns + %d aggregates exceed the window's %d columns", nsrc,
+                         r->group_nagg, kMaxProj);
+            if ((r->want & (MBC_WANT_POSITIONS | MBC_WANT_COLUMNS)) != (MBC_WANT_POSITIONS | MBC_WANT_COLUMNS))
+                MBC_FAIL(MBC_ERR_ARG, "mbc_shard_gather: a grouped result needs MBC_WANT_POSITIONS | MBC_WANT_COLUMNS");
+            for (int a = 0; a < r->group_nagg; ++a) {
+                src[nsrc] = r->d_aggs + (size_t)a * r->count;
+                src_stride[nsrc++] = 8;
+            }
+            own_count = true;
+            break;
+        }
+        default:
+            MBC_FAIL(MBC_ERR_ARG, "mbc_shard_gather: only scan, sorted, top-k and grouped results can be gathered (not a join's pairs)");
+    }
+    if (nsrc != s->ncols) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_gather: result has %d columns, window %d", nsrc, s->ncols);
     for (int c = 0; c < s->ncols; ++c)
-        if (r->cols[c].stride != s->strides[c]) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_gather: column %d stride %d, window %d", c, r->cols[c].stride, s->strides[c]);
+        if (src_stride[c] != s->strides[c]) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_gather: column %d stride %d, window %d", c, src_stride[c], s->strides[c]);
     mbc_ctx* ctx = s->ctx;
     MBC_CUDA(cudaSetDevice(ctx->device));
     const unsigned long long epoch = ++s->epoch;
@@ -391,13 +458,13 @@ int32_t mbc_shard_gather(mbc_shard* s, const mbc_result* r, int32_t beside_next_
     p.rank = s->rank;
     p.world = s->world;
     p.epoch = epoch;
-    p.my_aggs = reinterpret_cast<const unsigned long long*>(r->d_aggs);
+    p.my_aggs = own_count ? s->d_count_block : reinterpret_cast<const unsigned long long*>(r->d_aggs);
     p.cap_rows = s->cap_rows;
     p.src_pos = r->d_pos;
     p.dst_pos = reinterpret_cast<int64_t*>(s->win + s->off_pos[slot]);
     p.ncols = s->ncols;
     for (int c = 0; c < s->ncols; ++c) {
-        p.src[c] = r->cols[c].d;
+        p.src[c] = src[c];
         p.dst[c] = s->win + s->off_col[slot][c];
         p.stride[c] = s->strides[c];
     }
@@ -413,6 +480,12 @@ int32_t mbc_shard_gather(mbc_shard* s, const mbc_result* r, int32_t beside_next_
             MBC_CUDA(cudaStreamWaitEvent(s->side, s->ev_scan, 0));
         }
         st = s->side;
+    }
+    if (own_count) {
+        unsigned long long blk[kMaxAgg + 1] = {0};
+        blk[kMaxAgg] = (unsigned long long)r->count;
+        MBC_CUDA(cudaStreamWaitEvent(st, s->ev_push, 0));           // the previous step's publish has read the block
+        MBC_CUDA(cudaMemcpyAsync(s->d_count_block, blk, sizeof(blk), cudaMemcpyHostToDevice, st));
     }
     shard_publish_kernel<<<1, 32, 0, st>>>(p.ctl, s->rank, epoch, p.my_aggs);
     ctx->launches++;
@@ -459,6 +532,7 @@ int32_t mbc_shard_fence(mbc_shard* s) {
 int32_t mbc_shard_collect(mbc_shard* s, int64_t* total_rows, int64_t* rank_counts) {
     if (!s || !s->owned) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_collect: only the window's owner collects");
     if (s->epoch == 0) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_collect: nothing was gathered");
+    s->collected = 0;
     mbc_ctx* ctx = s->ctx;
     MBC_CUDA(cudaSetDevice(ctx->device));
     const int slot = (int)(s->epoch % kShardSlots);
@@ -480,6 +554,7 @@ int32_t mbc_shard_collect(mbc_shard* s, int64_t* total_rows, int64_t* rank_count
     }
     if (total_rows) *total_rows = s->total;
     if (s->dropped) MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_shard_collect: %lld rows did not fit the window of %lld rows", (long long)s->dropped, (long long)s->cap_rows);
+    s->collected = s->epoch;
     return MBC_OK;
 }
 
@@ -535,9 +610,140 @@ int32_t mbc_shard_read(mbc_shard* s, int32_t col, int64_t first_row, int64_t nro
 int32_t mbc_shard_release(mbc_shard* s) {
     if (!s || !s->owned || s->epoch == 0) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_release: only the window's owner releases a gathered step");
     MBC_CUDA(cudaSetDevice(s->ctx->device));
+    s->collected = 0;
     shard_release_kernel<<<1, 32, 0, s->side>>>(reinterpret_cast<ShardHeader*>(s->win), s->epoch);   // after the reads of the step
     s->ctx->launches++;
     MBC_CUDA(cudaGetLastError());
+    return MBC_OK;
+}
+
+int32_t mbc_shard_topk(mbc_shard* s, const mbc_coldesc* descs, const int32_t* key_fields, int32_t nkeys, int32_t descending, int64_t k,
+                       const int32_t* proj_fields, int32_t nproj, uint32_t want, mbc_result** out) {
+    if (!out || !descs || !key_fields || nkeys <= 0 || nproj < 0 || (nproj > 0 && !proj_fields)) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_topk: bad argument");
+    *out = nullptr;
+    MBC_TRY(merge_check(s, "mbc_shard_topk"));
+    if (k < 0) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_topk: k = %lld is negative", (long long)k);
+    if (want & (MBC_WANT_AGG | MBC_WANT_BITMAP))
+        MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_shard_topk: MBC_WANT_AGG / MBC_WANT_BITMAP are not available for a top-k");
+    if (nkeys > kMaxTerms || nproj > kMaxProj) MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_shard_topk: %d key fields / %d projected fields", nkeys, nproj);
+    Column cols[kMaxProj];
+    for (int c = 0; c < s->ncols; ++c) MBC_TRY(window_column(s, "mbc_shard_topk", c, descs[c], &cols[c]));
+    for (int q = 0; q < nkeys; ++q)
+        if (key_fields[q] < 0 || key_fields[q] >= s->ncols) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_topk: key field %d of %d", key_fields[q], s->ncols);
+    for (int c = 0; c < nproj; ++c)
+        if (proj_fields[c] < 0 || proj_fields[c] >= s->ncols) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_topk: projected field %d of %d", proj_fields[c], s->ncols);
+    mbc_ctx* ctx = s->ctx;
+    MBC_CUDA(cudaSetDevice(ctx->device));
+    const int64_t n = s->total, m = std::min<int64_t>(k, n);
+    const int64_t* win_pos = reinterpret_cast<const int64_t*>(s->win + s->off_pos[s->epoch % kShardSlots]);
+    begin_timing(ctx);
+    mbc_result* r = new mbc_result();
+    r->kind = mbc_result::kRows;
+    r->ctx = ctx;
+    ctx_retain(ctx);
+    r->want = want;
+    r->nrows = n;
+    r->count = m;
+    r->capacity = m;
+    uint32_t *rows = nullptr, *keys = nullptr, *bits = nullptr;
+    auto release = [&]() {
+        for (void* p : {(void*)rows, (void*)keys, (void*)bits}) dev_free(ctx, p);
+    };
+    auto fail = [&](int32_t st) {
+        release();
+        cudaStreamSynchronize(ctx->stream);                           // nothing reads the window after the call returns
+        mbc_result_free(r);
+        return st;
+    };
+#define MTRY(x) do { int32_t _s = (x); if (_s != MBC_OK) return fail(_s); } while (0)
+    // `rows` ends up holding the window rows in key order; the result is its first m
+    if (m > 0) {
+        MTRY(dev_alloc(ctx, (void**)&rows, (size_t)n * 4, false));
+        MTRY(dev_alloc(ctx, (void**)&keys, (size_t)n * 4, false));
+        MTRY(dev_alloc(ctx, (void**)&bits, 8, false));
+        sort_iota_kernel<<<merge_grid(ctx, n), 256, 0, ctx->stream>>>(n, rows);
+        ctx->launches++;
+        for (int q = nkeys - 1; q >= 0; --q) MTRY(sort_rows_by_column(ctx, rows, n, cols[key_fields[q]], descending != 0, keys, bits));
+    }
+    if ((want & MBC_WANT_POSITIONS) && m > 0) {
+        MTRY(dev_alloc(ctx, (void**)&r->d_pos, (size_t)m * 8, false));
+        sort_gather_kernel<<<merge_grid(ctx, m), 256, 0, ctx->stream>>>(rows, m, win_pos, 8, r->d_pos);
+        ctx->launches++;
+    }
+    if ((want & (MBC_WANT_COLUMNS | MBC_WANT_TUPLES)) && nproj > 0) {
+        for (int c = 0; c < nproj; ++c) {
+            const Column& col = cols[proj_fields[c]];
+            mbc_result::Col rc{col.type, col.width, col.stride, nullptr, nullptr};
+            MTRY(dev_alloc(ctx, &rc.d, (size_t)std::max<int64_t>(m, 1) * col.stride, false));
+            r->cols.push_back(rc);
+            if (m > 0) {
+                sort_gather_kernel<<<merge_grid(ctx, m), 256, 0, ctx->stream>>>(rows, m, col.d, col.stride, rc.d);
+                ctx->launches++;
+            }
+        }
+    }
+    end_timing(ctx);
+    if (cudaGetLastError() != cudaSuccess) return fail((set_error("mbc_shard_topk: launch failed"), MBC_ERR_CUDA));
+    MTRY(finish_result_host(r));
+#undef MTRY
+    if (cudaStreamSynchronize(ctx->stream) != cudaSuccess) return fail((set_error("mbc_shard_topk: merge failed"), MBC_ERR_CUDA));
+    release();
+    *out = r;
+    return MBC_OK;
+}
+
+int32_t mbc_shard_group(mbc_shard* s, const mbc_coldesc* key_descs, int32_t nkeys, const int32_t* agg_kinds, const int32_t* agg_types,
+                        int32_t nagg, uint32_t want, mbc_result** out) {
+    if (!out || !key_descs || nkeys <= 0 || nagg < 0 || (nagg > 0 && (!agg_kinds || !agg_types)))
+        MBC_FAIL(MBC_ERR_ARG, "mbc_shard_group: bad argument");
+    *out = nullptr;
+    MBC_TRY(merge_check(s, "mbc_shard_group"));
+    if (want & (MBC_WANT_TUPLES | MBC_WANT_BITMAP))
+        MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_shard_group: MBC_WANT_TUPLES / MBC_WANT_BITMAP are not available for groups");
+    if (nkeys + nagg > kMaxProj || nagg > kMaxAgg)
+        MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_shard_group: %d key columns + %d aggregates (max %d columns, %d aggregates)", nkeys, nagg, kMaxProj, kMaxAgg);
+    if (s->ncols != nkeys + nagg)
+        MBC_FAIL(MBC_ERR_ARG, "mbc_shard_group: %d key columns + %d aggregates for a window of %d columns", nkeys, nagg, s->ncols);
+    Column keys[kMaxProj];
+    for (int c = 0; c < nkeys; ++c) MBC_TRY(window_column(s, "mbc_shard_group", c, key_descs[c], &keys[c]));
+    const int slot = (int)(s->epoch % kShardSlots);
+    GroupAggSpec specs[kMaxAgg] = {};
+    for (int a = 0; a < nagg; ++a) {
+        const int kind = agg_kinds[a], type = agg_types[a];
+        if (kind < MBC_AGG_COUNT || kind > MBC_AGG_MAX) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_group: aggregate %d: unknown kind %d", a, kind);
+        if (kind != MBC_AGG_COUNT && type == MBC_ATTR_STRING) MBC_FAIL(MBC_ERR_UNSUPPORTED, "mbc_shard_group: aggregate %d over a string column", a);
+        if (kind != MBC_AGG_COUNT && type != MBC_ATTR_INTEGER && type != MBC_ATTR_REAL)
+            MBC_FAIL(MBC_ERR_ARG, "mbc_shard_group: aggregate %d: column type %d", a, type);
+        if (s->strides[nkeys + a] != 8) MBC_FAIL(MBC_ERR_ARG, "mbc_shard_group: window column %d (aggregate %d) has stride %d, not 8", nkeys + a, a, s->strides[nkeys + a]);
+        specs[a].kind = kind;
+        specs[a].type = kind == MBC_AGG_COUNT ? MBC_ATTR_INTEGER : type;
+        specs[a].src = s->win + s->off_col[slot][nkeys + a];
+    }
+    mbc_ctx* ctx = s->ctx;
+    MBC_CUDA(cudaSetDevice(ctx->device));
+    const int64_t n = s->total;
+    begin_timing(ctx);
+    mbc_result* r = new mbc_result();
+    r->ctx = ctx;
+    ctx_retain(ctx);
+    r->want = want;
+    r->nrows = n;
+    uint32_t* rows = nullptr;
+    int32_t st = dev_alloc(ctx, (void**)&rows, (size_t)std::max<int64_t>(n, 1) * 4, false);
+    if (st == MBC_OK && n > 0) {
+        sort_iota_kernel<<<merge_grid(ctx, n), 256, 0, ctx->stream>>>(n, rows);
+        ctx->launches++;
+    }
+    // the partials of one group keep rank order through the stable sort, so the fold's association is fixed
+    if (st == MBC_OK)
+        st = group_rows(ctx, rows, n, keys, nkeys, specs, nagg, true, reinterpret_cast<const int64_t*>(s->win + s->off_pos[slot]), 0, r);
+    dev_free(ctx, rows);
+    if (st != MBC_OK) {
+        cudaStreamSynchronize(ctx->stream);                           // nothing reads the window after the call returns
+        mbc_result_free(r);
+        return st;
+    }
+    *out = r;
     return MBC_OK;
 }
 

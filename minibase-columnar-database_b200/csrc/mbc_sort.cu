@@ -51,6 +51,10 @@ __global__ void __launch_bounds__(256) sort_rows_from_positions_kernel(const int
         rows[i] = (uint32_t)(pos[i] - base);
 }
 
+__global__ void __launch_bounds__(256) sort_iota_kernel(int64_t n, uint32_t* __restrict__ rows) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) rows[i] = (uint32_t)i;
+}
+
 __global__ void __launch_bounds__(256) sort_positions_kernel(const uint32_t* __restrict__ rows, int64_t n, int64_t base, int64_t* __restrict__ pos) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
         pos[i] = base + rows[i];
@@ -114,6 +118,7 @@ extern "C" int32_t mbc_sort(mbc_table* t, const int32_t* key_cols, int32_t nkeys
     const int64_t n = all->count;
 
     mbc_result* r = new mbc_result();
+    r->kind = mbc_result::kRows;
     r->ctx = ctx;
     ctx_retain(ctx);
     r->want = want;

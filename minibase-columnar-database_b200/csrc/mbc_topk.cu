@@ -279,6 +279,7 @@ extern "C" int32_t mbc_topk(mbc_table* t, const mbc_term* terms, int32_t nterms,
     begin_timing(ctx);
 
     mbc_result* r = new mbc_result();
+    r->kind = mbc_result::kRows;
     r->ctx = ctx;
     ctx_retain(ctx);
     r->want = want;

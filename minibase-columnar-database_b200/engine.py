@@ -421,7 +421,11 @@ class Shard:
     Same process (one host driving several GPUs):    root = Shard(ctx0, 0, n); root.create_window(...);
                                                      peer = Shard(ctx1, 1, n); peer.attach(root)
     One process per GPU: the root's `create_window` returns 64 handle bytes that the host ships to the peers by any
-    channel (torch.distributed broadcast in bench.py; a socket or a file in a JVM), and the peers `open_window(handle)`."""
+    channel (torch.distributed broadcast in bench.py; a socket or a file in a JVM), and the peers `open_window(handle)`.
+
+    Besides scans, the ranks may gather the results of `Table.top_k` / `Table.sort` (into a window shaped like their
+    projection) and of `Table.group_aggregate` (into a `create_group_window`); the root then merges them with `top_k` /
+    `group_aggregate` after `collect`."""
 
     def __init__(self, ctx: Context, rank: int, world: int):
         self.ctx, self.rank, self.world = ctx, rank, world
@@ -441,8 +445,8 @@ class Shard:
         except Exception:
             pass
 
-    def _strides(self, proj_descs):
-        st = [device_stride(d) for d in proj_descs]
+    def _strides(self, proj_descs, nagg: int = 0):
+        st = [device_stride(d) for d in proj_descs] + [8] * nagg
         return (C.c_int32 * max(len(st), 1))(*st), len(st)
 
     def create_window(self, capacity_rows: int, proj_descs: Sequence[tuple]) -> bytes:
@@ -450,6 +454,14 @@ class Shard:
         handle = (C.c_uint8 * N.IPC_HANDLE_BYTES)()
         N.check(N.lib().mbc_shard_window_create(self._h, capacity_rows, n, arr, handle))
         self.proj_descs, self.capacity = list(proj_descs), capacity_rows
+        return bytes(handle)
+
+    def create_group_window(self, capacity_groups: int, key_descs: Sequence[tuple], nagg: int) -> bytes:
+        """A window for the results of Table.group_aggregate: the key columns, then one 8-byte column per aggregate."""
+        arr, n = self._strides(key_descs, nagg)
+        handle = (C.c_uint8 * N.IPC_HANDLE_BYTES)()
+        N.check(N.lib().mbc_shard_window_create(self._h, capacity_groups, n, arr, handle))
+        self.proj_descs, self.capacity = list(key_descs), capacity_groups
         return bytes(handle)
 
     def open_window(self, handle: bytes, capacity_rows: int, proj_descs: Sequence[tuple]) -> None:
@@ -502,3 +514,30 @@ class Shard:
 
     def release(self) -> None:
         N.check(N.lib().mbc_shard_release(self._h))
+
+    def top_k(self, descs: Sequence[tuple], key_fields: Sequence[int], k: int, descending: bool = False,
+              proj_fields: Sequence[int] = (), want: int = N.WANT_POSITIONS | N.WANT_COLUMNS | N.WANT_HOST) -> "Result":
+        """Root, after collect: ORDER BY the window fields key_fields LIMIT k over the rows the ranks gathered from
+        Table.top_k (or Table.sort).  descs: (type, width) of every window column.  Same contract as Table.top_k over the
+        whole sharded table; positions are global."""
+        darr = (N.mbc_coldesc * max(len(descs), 1))(*[N.mbc_coldesc(int(t), int(w)) for t, w in descs])
+        karr = (C.c_int32 * max(len(key_fields), 1))(*key_fields)
+        parr = (C.c_int32 * max(len(proj_fields), 1))(*proj_fields)
+        h = C.c_void_p()
+        N.check(N.lib().mbc_shard_topk(self._h, darr, karr, len(key_fields), 1 if descending else 0, k, parr, len(proj_fields),
+                                       want, C.byref(h)))
+        return Result(self.ctx, h, [descs[f] for f in proj_fields], want, 0)
+
+    def group_aggregate(self, key_descs: Sequence[tuple], agg_kinds: Sequence[int], agg_types: Sequence[int],
+                        want: int = N.WANT_COLUMNS | N.WANT_POSITIONS | N.WANT_AGG | N.WANT_HOST) -> "Result":
+        """Root, after collect: GROUP BY over the grouped results the ranks gathered (Table.group_aggregate with the same
+        keys and aggregates).  agg_kinds / agg_types: AGG_* kind and aggregated column type of each aggregate.  Same
+        contract as Table.group_aggregate over the whole sharded table."""
+        darr = (N.mbc_coldesc * max(len(key_descs), 1))(*[N.mbc_coldesc(int(t), int(w)) for t, w in key_descs])
+        karr = (C.c_int32 * max(len(agg_kinds), 1))(*agg_kinds)
+        tarr = (C.c_int32 * max(len(agg_types), 1))(*agg_types)
+        if len(agg_kinds) != len(agg_types):
+            raise ValueError(f"{len(agg_kinds)} aggregate kinds for {len(agg_types)} types")
+        h = C.c_void_p()
+        N.check(N.lib().mbc_shard_group(self._h, darr, len(key_descs), karr, tarr, len(agg_kinds), want, C.byref(h)))
+        return Result(self.ctx, h, list(key_descs), want, len(agg_kinds))
